@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the HesAffNet + HardNet detect-and-describe hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|5] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|5] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the whole path (pyramid -> Hessian/NMS -> top-k -> sample -> AffNet -> filter -> sample
 -> OriNet -> sample -> HardNet) over one batch of B synthetic images per GPU.  Headline workload (--config 2, the default):
@@ -74,6 +74,30 @@ def make_images(B, seed0, H, W):
 def load_state_dicts():
     from helpers import load_weights
     return load_weights()
+
+
+DUMP_BUDGET = 64_000_000     # bytes that --dump-outputs may write
+
+
+def dump_outputs(out_dir, lafs, resp, desc, count):
+    """--dump-outputs: what the timed path returned in its last step for this rank's images, as DIR/<name>.npy (float32; count as
+    float64), so that two builds can be compared output for output.  Rows at or past an image's count are unspecified, so they are
+    written as zeros.  Above DUMP_BUDGET only a fixed, seeded sample of keypoint slots is written (the same slots for every image;
+    their indices in keypoint_slots.npy)."""
+    B, K = resp.shape
+    valid = torch.arange(K)[None, :] < count.long()[:, None]
+    out = {"lafs": lafs.masked_fill(~valid[:, :, None, None], 0.0), "resp": resp.masked_fill(~valid, 0.0),
+           "desc": desc.masked_fill(~valid[:, :, None], 0.0)}
+    per_slot = B * (6 + 1 + 128) * 4                           # bytes of lafs, resp and desc per keypoint slot
+    slots = (DUMP_BUDGET - 8 * B - 4096) // (per_slot + 8)      # count.npy, keypoint_slots.npy and the .npy headers
+    if slots < K:
+        keep = np.sort(np.random.default_rng(0).choice(K, slots, replace=False))
+        out = {k: a[:, torch.from_numpy(keep)] for k, a in out.items()}
+        out["keypoint_slots"] = keep.astype(np.float64)
+    out["count"] = count.double()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a.numpy() if isinstance(a, torch.Tensor) else a))
 
 
 class ClockSampler:
@@ -258,7 +282,9 @@ class Workload:
     def step_device(self):
         return self._run(self.dev_imgs)
 
-    def timed(self, steps, warmup, sampler=None):
+    def timed(self, steps, warmup, sampler=None, keep_last=False):
+        """keep_last: copy the last timed step's outputs to host memory as self.last_host (after the timed region, before the clock
+        sampler's extra steps overwrite the pipeline's buffers)."""
         ctx = self.ctx
         dist, dev, flush = ctx["dist"], ctx["dev"], ctx["flush"]
         for _ in range(warmup):
@@ -280,6 +306,8 @@ class Workload:
             evs.append((e0, e1))
         torch.cuda.synchronize()
         t_stop = time.time()
+        if keep_last:
+            self.last_host = [t.cpu() for t in self.last]
         clocks = None
         if sampler:
             # The sampler runs since before the warm-up; only samples that arrived inside the timed region count.  If the region was
@@ -410,7 +438,12 @@ def _main(real_stdout):
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra configurations (B=1, B=64, configs 3 and 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's images) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
@@ -448,8 +481,9 @@ def _main(real_stdout):
     wl = Workload(ctx, H, W, K, border, B, use_graph)
     pipe = wl.pipe
 
-    total_ms, clocks = wl.timed(args.steps, args.warmup, sampler)
+    total_ms, clocks = wl.timed(args.steps, args.warmup, sampler, keep_last=bool(args.dump_outputs))
     pipe.check()
+    last_outputs = wl.last_host if args.dump_outputs else None
     wl.check_exchange()
     n_desc = int(wl.last[3].sum().item())
     e2e_ms = wl.timed_e2e(args.steps, args.warmup)
@@ -554,6 +588,8 @@ def _main(real_stdout):
             line["extra"] = extra
         if exchange_cost is not None:
             line["exchange"] = exchange_cost
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, *last_outputs)
         emit(real_stdout, line)
     if dist is not None:
         dist.destroy_process_group()

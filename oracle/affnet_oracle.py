@@ -8,8 +8,7 @@ This is an independent restatement (plain PyTorch-CPU / numpy, fp32 unless noted
 the reference (ducha-aiki/affnet @ da7cf51) executes under Python 3 / torch 2.x.  Every function
 cites the reference file:line it follows.  Parity is PINNED: `tests/golden/make_golden.py` ran the
 unmodified reference in the build container and committed its outputs under `tests/golden/`;
-`tests/test_oracle_golden.py` checks this oracle against them (and against the live reference when
-`/root/reference` is present).
+`tests/test_oracle_golden.py` checks this oracle against them.
 
 Quirks reproduced on purpose (SURVEY.md §8a Q1-Q8): non-integer Gaussian tap spacing (Q1), the
 +0.5 px soft-argmax bias (Q2), uint8 wrap of the octave map (Q4), mixed units in the boundary

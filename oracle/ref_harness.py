@@ -1,7 +1,7 @@
 """Harness that imports the UNMODIFIED reference (ducha-aiki/affnet) from $AFFNET_REF, /root/reference or
 baseline/_ref (first that holds SparseImgRepresenter.py) on CPU.  TEST INFRASTRUCTURE ONLY: used by
-`tests/golden/make_golden.py` to generate golden vectors and by `-m "not gpu"` tests (when the
-reference tree is present) to pin `oracle/affnet_oracle.py`.  Never imported by the product.
+`tests/golden/make_golden.py` to generate the golden vectors that pin `oracle/affnet_oracle.py`, and by
+bench.py's CPU leg when the reference tree is present.  Never imported by the product.
 
 Shims (no edits to the reference): matplotlib stub (LAF.py:2 imports pyplot), map_location='cpu'
 for checkpoints saved from CUDA, stdout silenced (the detector prints timings on every forward).

@@ -19,6 +19,7 @@ changes.  Outputs (all .npz, compressed):
   graf_match.npz     the reference's own application test (train_AffNet_test_on_graffity.py:262-300): graf img1 <-> img6, K=3000,
                      HardNet + SNN 0.8 + 6 px reprojection check, for hand-crafted orientation / OriNet / no orientation:
                      tentative and true match counts, img6 and H1to6p (`... make_golden.py match`)
+  distance.npz       Losses.distance_matrix_vector on seeded random descriptors (`... make_golden.py distance`)
 """
 import contextlib
 import io
@@ -226,6 +227,17 @@ def make_match():
     save("graf_match.npz", **out)
 
 
+def make_distance():
+    """8f row 3: Losses.distance_matrix_vector on 50 x 70 seeded random descriptors (inputs stored with the output)."""
+    import importlib
+    R.ref_modules()
+    LS = importlib.import_module("Losses")
+    g = torch.Generator().manual_seed(5)
+    a, b = torch.randn(50, 128, generator=g), torch.randn(70, 128, generator=g)
+    with torch.no_grad():
+        save("distance.npz", a=a, b=b, d=LS.distance_matrix_vector(a, b))
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "ell":
         make_ell()
@@ -233,8 +245,11 @@ if __name__ == "__main__":
         make_match()
     elif len(sys.argv) > 1 and sys.argv[1] == "jit":
         make_jit()
+    elif len(sys.argv) > 1 and sys.argv[1] == "distance":
+        make_distance()
     else:
         main()
         make_ell()
         make_match()
         make_jit()
+        make_distance()
