@@ -80,6 +80,7 @@ PROTOTYPES = {
     "ag_affnet_forward_raw": (i32, [vp, vp, i32, vp, vp, sz, vp]),
     "ag_orinet_forward_raw": (i32, [vp, vp, i32, vp, vp, sz, vp]),
     "ag_debug_pyramid_mode": (i32, [i32]),
+    "ag_debug_fuse_l3": (i32, [i32]),
     "ag_debug_tcx_layer": (i32, [vp, vp, i32, i32, vp, vp, sz, vp]),
     "ag_affnet_forward": (i32, [vp, vp, i32, vp, i32, vp, vp, sz, vp]),
     "ag_orinet_forward": (i32, [vp, vp, i32, vp, i32, vp, vp, vp, sz, vp]),

@@ -1,7 +1,8 @@
 // Second-generation tensor-core engine of AffNet / OriNet / HardNet (tcx_first.cuh, tcx_conv.cuh): row tiles without x padding, the
 // three taps of a kernel row stacked along N, x shifts by warp shuffles in the epilogue.  Replaces the conv stacks of
 // architectures.py:207-235 / 36-82 and HardNet.py:67-101 (BatchNorm folded, ReLU fused); the 8x8 heads stay the GEMM kernels of
-// tc_head.cuh (same head-operand layout).  Per net:  tcx_first_kernel (sampler + input_norm + conv1 + conv2)  ->  tcx_conv_kernel x4.
+// tc_head.cuh (same head-operand layout).  Per net:  tcx_first_kernel (sampler + input_norm + conv1 + conv2)  ->  tcx_conv_kernel x4;
+// AffNet / OriNet: conv3 inside tcx_first_kernel as well (AG_FUSE_L3), then tcx_conv_kernel x3.
 // Numerics: AffNet / OriNet with fp16 residual planes of weights and activations in every layer (three MMAs per K step, fp32-grade);
 // HardNet fp16 activations, weights with their fp16 residual in layers 2 and 3 (emulation on the 2000 graf patches: plain fp16 weights give a
 // descriptor error of 1.1e-3, dominated by the weight rounding of the early layers; measured on the GPU with the residuals of layers 2-3:
@@ -71,19 +72,23 @@ static int launch_conv(const void* in, void* out, const __half* w, const float* 
     return AG_OK;
 }
 
-template <int C1, int COUT, int SA, int SW, int OSA, int BF = 0>
-static int launch_first(void* out, const __half* w, const float* b, float inv_scale, int n, int group, const int* count, cudaStream_t st, const FirstSrc& src) {
-    using Cfg = XFirstCfg<C1, COUT, SA, SW, OSA>;
-    auto kern = tcx_first_kernel<C1, COUT, SA, SW, OSA, BF>;
+// L3 = 1: conv layer 3 fused (its weights / bias / scale in w3 / b3 / inv_scale3); it writes out3 and `out` is not used
+template <int C1, int COUT, int SA, int SW, int OSA, int BF = 0, int L3 = 0>
+static int launch_first(void* out, const __half* w, const float* b, float inv_scale, int n, int group, const int* count, cudaStream_t st, const FirstSrc& src,
+                        void* out3 = nullptr, const __half* w3 = nullptr, const float* b3 = nullptr, float inv_scale3 = 0.f) {
+    using Cfg = XFirstCfg<C1, COUT, SA, SW, OSA, L3>;
+    auto kern = tcx_first_kernel<C1, COUT, SA, SW, OSA, BF, L3>;
     static bool configured[64] = {};
     int rc = ensure_smem_attr((const void*)kern, (int)Cfg::SMEM, configured, "tcx_first smem attr");
     if (rc != AG_OK) return rc;
     XArgs a;
     a.in = nullptr; a.out = out; a.wpk = w; a.bias = b; a.inv_scale = inv_scale; a.n = n; a.group = group; a.count = count; a.prof_id = 0;
+    XArgs a3 = a;
+    a3.out = out3; a3.wpk = w3; a3.bias = b3; a3.inv_scale = inv_scale3;
     int gx = num_sms();
     if (gx > n) gx = n;
     if (gx < 1) gx = 1;
-    kern<<<gx, Cfg::THREADS, Cfg::SMEM, st>>>(a, src);
+    kern<<<gx, Cfg::THREADS, Cfg::SMEM, st>>>(a, src, a3);
     AG_CHECK_LAUNCH("tcx_first_kernel");
     return AG_OK;
 }
@@ -212,6 +217,14 @@ static inline int tcx_lox(const ag_net* net) { return ((net->kind == AG_NET_AFFN
 #ifndef AG_AFF_EW4
 #define AG_AFF_EW4 8   // layer 4 waited for its 4-warp epilogue 23 % of the time: 0.72 -> 0.61 ms (AffNet), 0.48 -> 0.41 (OriNet); layer 3 is HBM bound (no change)
 #endif
+// Conv layer 3 fused into the first kernel (tcx_first.cuh, L3 = 1): layer 2's output stays in shared memory instead of a 64 KiB per
+// patch round trip through HBM, and the step has one launch fewer per net.  Bit-identical to the unfused pair (tests/test_gpu_fused_l3.py).
+// AG_FUSE_L3=0 builds with the unfused pair as the default; ag_debug_fuse_l3() switches at run time.  The byte residual planes
+// (AG_AFF_LO8 / AG_ORI_LO8) only exist to shrink that HBM round trip: a net built with them runs the unfused pair.
+#ifndef AG_FUSE_L3
+#define AG_FUSE_L3 1
+#endif
+static int g_tcx_fuse_l3 = AG_FUSE_L3;
 template <int LOX>
 static int trunk_affori_t(const ag_net* net, const tc::FirstSrc& src0, int n, int group, const int* count, void* bufA, void* bufB, void* feat,
                           cudaStream_t st, int upto) {
@@ -219,9 +232,15 @@ static int trunk_affori_t(const ag_net* net, const tc::FirstSrc& src0, int n, in
     tc::FirstSrc src = src0;
     src.w1 = net->d_w1; src.b1 = net->d_b[0]; src.w1_inv = net->w_inv_scale[0]; src.w1_scale = 1.0f / net->w_inv_scale[0];
     int rc;
-    if ((rc = launch_first<16, 16, 1, 1, LOX>(bufB, net->d_wx[1], net->d_b[1], net->w_inv_scale[1], n, group, count, st, src))) return rc;
-    if (upto <= 2) return AG_OK;
-    if ((rc = launch_conv<16, 32, 32, 2, 1, 3, L_S1_16, LOX, 1, 1, AG_AFF_EW3>(bufB, bufA, net->d_wx[2], net->d_b[2], net->w_inv_scale[2], n, group, count, st))) return rc;
+    if (LOX == 1 && g_tcx_fuse_l3 && upto >= 3) {   // layer 2's output only exists on the unfused path (upto = 2)
+        if ((rc = launch_first<16, 16, 1, 1, 1, 0, 1>(nullptr, net->d_wx[1], net->d_b[1], net->w_inv_scale[1], n, group, count, st, src, bufA, net->d_wx[2],
+                                                      net->d_b[2], net->w_inv_scale[2])))
+            return rc;
+    } else {
+        if ((rc = launch_first<16, 16, 1, 1, LOX>(bufB, net->d_wx[1], net->d_b[1], net->w_inv_scale[1], n, group, count, st, src))) return rc;
+        if (upto <= 2) return AG_OK;
+        if ((rc = launch_conv<16, 32, 32, 2, 1, 3, L_S1_16, LOX, 1, 1, AG_AFF_EW3>(bufB, bufA, net->d_wx[2], net->d_b[2], net->w_inv_scale[2], n, group, count, st))) return rc;
+    }
     if (upto <= 3) return AG_OK;
     if ((rc = launch_conv<32, 32, 16, 1, 1, 4, L_S2_8P, 1, 1, 1, AG_AFF_EW4>(bufA, bufB, net->d_wx[3], net->d_b[3], net->w_inv_scale[3], n, group, count, st))) return rc;
     if (upto <= 4) return AG_OK;
@@ -291,6 +310,14 @@ int ag_debug_tcx_layer(const ag_net_t* net, const float* d_patches, int n, int u
     tcx::tcx_decode_kernel<<<296, 256, 0, st>>>((const __half*)buf, lay, C, osa, H, n, d_out);
     AG_CHECK_LAUNCH("tcx_decode_kernel");
     return AG_OK;
+}
+
+// Developer switch: 1 = conv layer 3 of AffNet / OriNet fused into the first kernel (default unless built with AG_FUSE_L3=0), 0 = the
+// unfused pair.  Returns the previous mode.
+int ag_debug_fuse_l3(int fused) {
+    const int old = g_tcx_fuse_l3;
+    g_tcx_fuse_l3 = fused ? 1 : 0;
+    return old;
 }
 
 }  // extern "C"

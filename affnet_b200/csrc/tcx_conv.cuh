@@ -137,6 +137,43 @@ struct XIn {
     static_assert(!(STRIDE == 1 && H == 32), "the 32x32 stride-1 layer lives in tcx_first.cuh");
 };
 
+// MMAs of one stride-2 output tile (M = 128) into accumulator columns d .. d + 3 NT: for kernel row dy and 16 input channels the odd-x
+// plane (taps dx = 0 | 2, N = 2 NT, columns d .. d + 2 NT) and the even-x plane (tap dx = 1, N = NT, columns d + 2 NT ..), each as the
+// A_hi W_hi, A_hi W_lo (SW) and A_lo W_hi (SA) products.  a_t: the tile's first slot of the stage (16-byte units), PL / RW: plane and
+// row slots, GS: slots per channel group; w_base: the layer's weight blocks (16-byte units).  Shared by tcx_conv_kernel and the fused
+// layer 3 of tcx_first_kernel, so both issue the same MMAs in the same order.
+template <int KC, int NT, int PL, int RW, int GS, int SA, int SW, int BF>
+__device__ __forceinline__ void xmma_s2_tile(uint32_t d, uint32_t a_t, uint32_t w_base) {
+    constexpr uint32_t idesc2 = XFmt<BF>::IDESC | (1u << 4) | ((uint32_t)((2 * NT) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    constexpr uint32_t idesc1 = XFmt<BF>::IDESC | (1u << 4) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    constexpr int NRO = (1 + SW) * 2 * NT, NRE = (1 + SW) * NT;   // weight rows per K group: odd-x plane [hi: dx0 dx2][lo: ...], even-x plane [hi: dx1][lo: dx1]
+    constexpr uint32_t LBO_A = ((uint32_t)GS) << 16;
+#pragma unroll
+    for (int dy = 0; dy < 3; dy++) {
+        const int py = (dy == 1) ? 0 : 1, ro = (dy == 0) ? 0 : 1;
+#pragma unroll
+        for (int j = 0; j < KC / 2; j++) {
+            const uint32_t blk = w_base + (uint32_t)((dy * (KC / 2) + j) * 2 * (NRO + NRE));
+            const uint32_t bo_hi = (blk & 0x3FFFu) | ((uint32_t)NRO << 16), bo_lo = ((blk + 2 * NT) & 0x3FFFu) | ((uint32_t)NRO << 16);
+            const uint32_t be = blk + 2 * NRO;
+            const uint32_t be_hi = (be & 0x3FFFu) | ((uint32_t)NRE << 16), be_lo = ((be + NT) & 0x3FFFu) | ((uint32_t)NRE << 16);
+            // odd-x plane (px = 1): taps dx = 0 and dx = 2
+            const uint32_t ao = a_t + (uint32_t)((py * 2 + 1) * PL + ro * RW);
+            const uint32_t ao_hi = ((ao + (uint32_t)(2 * j * GS)) & 0x3FFFu) | LBO_A, ao_lo = ((ao + (uint32_t)((KC + 2 * j) * GS)) & 0x3FFFu) | LBO_A;
+            if (dy == 0 && j == 0) umma_f16_lo<0>(d, ao_hi, bo_hi, idesc2); else umma_f16_lo<1>(d, ao_hi, bo_hi, idesc2);
+            if (SW) umma_f16_lo<1>(d, ao_hi, bo_lo, idesc2);
+            if (SA) umma_f16_lo<1>(d, ao_lo, bo_hi, idesc2);
+            // even-x plane (px = 0): tap dx = 1
+            const uint32_t ae = a_t + (uint32_t)((py * 2 + 0) * PL + ro * RW);
+            const uint32_t ae_hi = ((ae + (uint32_t)(2 * j * GS)) & 0x3FFFu) | LBO_A, ae_lo = ((ae + (uint32_t)((KC + 2 * j) * GS)) & 0x3FFFu) | LBO_A;
+            const uint32_t de = d + (uint32_t)(2 * NT);
+            if (dy == 0 && j == 0) umma_f16_lo<0>(de, ae_hi, be_hi, idesc1); else umma_f16_lo<1>(de, ae_hi, be_hi, idesc1);
+            if (SW) umma_f16_lo<1>(de, ae_hi, be_lo, idesc1);
+            if (SA) umma_f16_lo<1>(de, ae_lo, be_hi, idesc1);
+        }
+    }
+}
+
 struct XArgs {
     const __half* in;     // HBM activation buffer in the layer's input layout
     void* out;            // next layer's buffer
@@ -266,8 +303,6 @@ __global__ void __launch_bounds__(64 + 32 * EW + (SA == 2 ? 128 : 0), 1) tcx_con
     } else if (warp == EW + 1) {
         // ===== MMA issuer (warp-uniform control flow, one elected lane issues) =====
         constexpr uint32_t idesc3 = XFmt<BF>::IDESC | (1u << 4) | ((uint32_t)((3 * NT) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-        constexpr uint32_t idesc2 = XFmt<BF>::IDESC | (1u << 4) | ((uint32_t)((2 * NT) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-        constexpr uint32_t idesc1 = XFmt<BF>::IDESC | (1u << 4) | ((uint32_t)(NT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
         const uint32_t leader = elect_one();
         mbar_wait(wbar, 0);
         tc_fence_after();
@@ -305,31 +340,7 @@ __global__ void __launch_bounds__(64 + 32 * EW + (SA == 2 ? 128 : 0), 1) tcx_con
                             }
                         }
                     } else {
-#pragma unroll
-                        for (int dy = 0; dy < 3; dy++) {
-                            constexpr int PL = In::PLANE;
-                            const int py = (dy == 1) ? 0 : 1, ro = (dy == 0) ? 0 : 1;
-#pragma unroll
-                            for (int j = 0; j < KC / 2; j++) {
-                                const uint32_t blk = w_base + (uint32_t)((dy * (KC / 2) + j) * 2 * (Cfg::NRO + Cfg::NRE));
-                                const uint32_t bo_hi = (blk & 0x3FFFu) | ((uint32_t)Cfg::NRO << 16), bo_lo = ((blk + 2 * NT) & 0x3FFFu) | ((uint32_t)Cfg::NRO << 16);
-                                const uint32_t be = blk + 2 * Cfg::NRO;
-                                const uint32_t be_hi = (be & 0x3FFFu) | ((uint32_t)Cfg::NRE << 16), be_lo = ((be + NT) & 0x3FFFu) | ((uint32_t)Cfg::NRE << 16);
-                                // odd-x plane (px = 1): taps dx = 0 and dx = 2
-                                const uint32_t ao = a_t + (uint32_t)((py * 2 + 1) * PL + ro * RW);
-                                const uint32_t ao_hi = ((ao + (uint32_t)(2 * j * GS)) & 0x3FFFu) | LBO_A, ao_lo = ((ao + (uint32_t)((KC + 2 * j) * GS)) & 0x3FFFu) | LBO_A;
-                                if (dy == 0 && j == 0) umma_f16_lo<0>(d, ao_hi, bo_hi, idesc2); else umma_f16_lo<1>(d, ao_hi, bo_hi, idesc2);
-                                if (SW) umma_f16_lo<1>(d, ao_hi, bo_lo, idesc2);
-                                if (SA) umma_f16_lo<1>(d, ao_lo, bo_hi, idesc2);
-                                // even-x plane (px = 0): tap dx = 1
-                                const uint32_t ae = a_t + (uint32_t)((py * 2 + 0) * PL + ro * RW);
-                                const uint32_t ae_hi = ((ae + (uint32_t)(2 * j * GS)) & 0x3FFFu) | LBO_A, ae_lo = ((ae + (uint32_t)((KC + 2 * j) * GS)) & 0x3FFFu) | LBO_A;
-                                const uint32_t de = d + (uint32_t)(2 * NT);
-                                if (dy == 0 && j == 0) umma_f16_lo<0>(de, ae_hi, be_hi, idesc1); else umma_f16_lo<1>(de, ae_hi, be_hi, idesc1);
-                                if (SW) umma_f16_lo<1>(de, ae_hi, be_lo, idesc1);
-                                if (SA) umma_f16_lo<1>(de, ae_lo, be_hi, idesc1);
-                            }
-                        }
+                        xmma_s2_tile<KC, NT, In::PLANE, RW, GS, SA, SW, BF>(d, a_t, w_base);
                     }
                     umma_commit(&tfull[ab]);
                 }

@@ -178,6 +178,10 @@ int ag_net_get_engine(const ag_net_t* net);
 /* Developer switch: 1 = ag_pyramid_build runs one launch per octave (pyramid_fused.cuh: bit-identical, measured slower), 0 = one
  * launch per level (default).  Returns the previous mode. */
 int ag_debug_pyramid_mode(int fused);
+/* Developer switch: 1 = conv layer 3 of AffNet / OriNet runs inside the first tcgen05 kernel (layer 2's output stays in shared memory;
+ * bit-identical; the default unless built with -DAG_FUSE_L3=0), 0 = first kernel and layer-3 kernel as two launches.  Returns the
+ * previous mode. */
+int ag_debug_fuse_l3(int fused);
 /* Developer diagnostic: run the second-generation trunk on materialised patches [n,32,32] up to conv layer `upto` (2..5) and decode
  * that layer's activations (fp16 hi [+ lo] planes in the engine's HBM layout) to fp32 [n,C,H,H].  d_ws: ag_net_workspace_bytes(). */
 int ag_debug_tcx_layer(const ag_net_t* net, const float* d_patches, int n, int upto, float* d_out, void* d_ws, size_t ws_bytes, void* stream);
