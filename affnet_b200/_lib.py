@@ -49,6 +49,14 @@ class PipelineConfig(C.Structure):
     ]
 
 
+SHAPE_AFFNET, SHAPE_BAUMBERG = 0, 1
+ORI_NONE, ORI_ORINET, ORI_HIST = 0, 1, 2
+
+
+class PipelineEstimators(C.Structure):
+    _fields_ = [("shape", C.c_int), ("num_Baum_iters", C.c_int), ("shape_ps", C.c_int), ("ori", C.c_int), ("ori_ps", C.c_int)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/affnet_b200.h
 vp, i32, f32, f64, sz = C.c_void_p, C.c_int, C.c_float, C.c_double, C.c_size_t
 PROTOTYPES = {
@@ -93,10 +101,13 @@ PROTOTYPES = {
     "ag_circular_gauss_kernel": (i32, [i32, f64, vp]),
     "ag_orientation_hist": (i32, [vp, i32, i32, vp, vp, vp]),
     "ag_baumberg_shape": (i32, [vp, i32, i32, vp, vp, vp]),
+    "ag_orientation_hist_pyr": (i32, [C.POINTER(PyramidPlan), vp, vp, vp, vp, vp, i32, i32, vp, vp, vp]),
+    "ag_baumberg_shape_pyr": (i32, [C.POINTER(PyramidPlan), vp, vp, vp, vp, vp, i32, i32, i32, vp, vp]),
     "ag_distance_matrix": (i32, [vp, i32, vp, i32, i32, vp, vp]),
     "ag_match_snn_workspace_bytes": (sz, [i32, i32]),
     "ag_match_snn": (i32, [vp, i32, vp, i32, i32, f32, vp, sz, vp, vp, vp, vp, vp]),
     "ag_pipeline_create": (i32, [C.POINTER(PipelineConfig), vp, vp, vp, C.POINTER(vp)]),
+    "ag_pipeline_create_ex": (i32, [C.POINTER(PipelineConfig), C.POINTER(PipelineEstimators), vp, vp, vp, C.POINTER(vp)]),
     "ag_pipeline_destroy": (None, [vp]),
     "ag_pipeline_workspace_bytes": (sz, [vp]),
     "ag_pipeline_plan": (C.POINTER(PyramidPlan), [vp]),

@@ -134,4 +134,41 @@ __device__ __forceinline__ void laf_sample_xy(const float* __restrict__ L, int h
     py = __fsub_rn(__fmaf_rn(a21, xj, __fmaf_rn(a22, yi, ty)), 0.5f);
 }
 
+// Pyramid geometry passed by value to the kernels that sample patches straight from the pyramid (row b*cap+i reads level
+// pyr[oct][lvl] of image b).
+struct PyrGeom {
+    int n_octaves, n_levels, B;
+    int h[AG_MAX_OCTAVES], w[AG_MAX_OCTAVES];
+    long long off[AG_MAX_OCTAVES][AG_MAX_LEVELS];
+};
+
+inline PyrGeom make_geom(const ag_pyramid_plan_t* p) {
+    PyrGeom g;
+    g.n_octaves = p->n_octaves; g.n_levels = p->n_levels; g.B = p->B;
+    for (int o = 0; o < AG_MAX_OCTAVES; o++) {
+        g.h[o] = p->h[o]; g.w[o] = p->w[o];
+        for (int l = 0; l < AG_MAX_LEVELS; l++) g.off[o][l] = p->level_offset[o][l];
+    }
+    return g;
+}
+
+// LAF_A <- LAF_A * R for R = [r0 r1; r2 r3] (getOrientation's compose, SparseImgRepresenter.py:175)
+__device__ __forceinline__ void laf_rotate(float (&l)[6], float r0, float r1, float r2, float r3) {
+    const float l00 = l[0], l01 = l[1], l10 = l[3], l11 = l[4];
+    l[0] = fmaf(l00, r0, l01 * r2); l[1] = fmaf(l00, r1, l01 * r3);
+    l[3] = fmaf(l10, r0, l11 * r2); l[4] = fmaf(l10, r1, l11 * r3);
+}
+
+// out = a * b for 2x2 matrices, in torch.bmm's fp32 operation order (row-by-column, two products added left to right)
+__device__ __forceinline__ void mat2_mul(const float (&a)[4], const float (&b)[4], float (&out)[4]) {
+    out[0] = __fmaf_rn(a[1], b[2], __fmul_rn(a[0], b[0])); out[1] = __fmaf_rn(a[1], b[3], __fmul_rn(a[0], b[1]));
+    out[2] = __fmaf_rn(a[3], b[2], __fmul_rn(a[2], b[0])); out[3] = __fmaf_rn(a[3], b[3], __fmul_rn(a[2], b[1]));
+}
+
+// out = [a * l[:, :2] | l[:, 2]] for a 2x2 matrix a and a LAF l (the bmm of SparseImgRepresenter.py:134-135)
+__device__ __forceinline__ void laf_left_mul(const float (&a)[4], const float (&l)[6], float (&out)[6]) {
+    out[0] = __fmaf_rn(a[1], l[3], __fmul_rn(a[0], l[0])); out[1] = __fmaf_rn(a[1], l[4], __fmul_rn(a[0], l[1])); out[2] = l[2];
+    out[3] = __fmaf_rn(a[3], l[3], __fmul_rn(a[2], l[0])); out[4] = __fmaf_rn(a[3], l[4], __fmul_rn(a[2], l[1])); out[5] = l[5];
+}
+
 }  // namespace ag

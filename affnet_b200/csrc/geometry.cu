@@ -116,9 +116,9 @@ __global__ void lafs_rotate_kernel(float* __restrict__ lafs, const float* __rest
     if (i >= n) return;
     float* L = lafs + (size_t)i * 6;
     const float* r = R + (size_t)i * 4;
-    const float l00 = L[0], l01 = L[1], l10 = L[3], l11 = L[4];
-    L[0] = fmaf(l00, r[0], l01 * r[2]); L[1] = fmaf(l00, r[1], l01 * r[3]);
-    L[3] = fmaf(l10, r[0], l11 * r[2]); L[4] = fmaf(l10, r[1], l11 * r[3]);
+    float l[6] = {L[0], L[1], 0.f, L[3], L[4], 0.f};
+    laf_rotate(l, r[0], r[1], r[2], r[3]);
+    L[0] = l[0]; L[1] = l[1]; L[3] = l[3]; L[4] = l[4];
 }
 
 __global__ void lafs_scale_kernel(const float* __restrict__ in, float* __restrict__ out, int n, float ac, float xc, float yc) {
@@ -163,19 +163,23 @@ namespace ag {
 __global__ void mat2_compose_kernel(const float* __restrict__ A, const float* __restrict__ B, float* __restrict__ out, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const float a0 = A[i * 4], a1 = A[i * 4 + 1], a2 = A[i * 4 + 2], a3 = A[i * 4 + 3];
-    const float b0 = B[i * 4], b1 = B[i * 4 + 1], b2 = B[i * 4 + 2], b3 = B[i * 4 + 3];
-    out[i * 4 + 0] = __fmaf_rn(a1, b2, __fmul_rn(a0, b0)); out[i * 4 + 1] = __fmaf_rn(a1, b3, __fmul_rn(a0, b1));
-    out[i * 4 + 2] = __fmaf_rn(a3, b2, __fmul_rn(a2, b0)); out[i * 4 + 3] = __fmaf_rn(a3, b3, __fmul_rn(a2, b1));
+    const float a[4] = {A[i * 4], A[i * 4 + 1], A[i * 4 + 2], A[i * 4 + 3]};
+    const float b[4] = {B[i * 4], B[i * 4 + 1], B[i * 4 + 2], B[i * 4 + 3]};
+    float o[4];
+    mat2_mul(a, b, o);
+#pragma unroll
+    for (int q = 0; q < 4; q++) out[i * 4 + q] = o[q];
 }
 // out = [A * L[:, :, :2] | L[:, :, 2]] : the working LAF of the next Baumberg iteration (SparseImgRepresenter.py:134-135)
 __global__ void lafs_left_multiply_kernel(const float* __restrict__ A, const float* __restrict__ Lf, float* __restrict__ out, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const float a0 = A[i * 4], a1 = A[i * 4 + 1], a2 = A[i * 4 + 2], a3 = A[i * 4 + 3];
-    const float l0 = Lf[i * 6], l1 = Lf[i * 6 + 1], l3 = Lf[i * 6 + 3], l4 = Lf[i * 6 + 4];
-    out[i * 6 + 0] = __fmaf_rn(a1, l3, __fmul_rn(a0, l0)); out[i * 6 + 1] = __fmaf_rn(a1, l4, __fmul_rn(a0, l1)); out[i * 6 + 2] = Lf[i * 6 + 2];
-    out[i * 6 + 3] = __fmaf_rn(a3, l3, __fmul_rn(a2, l0)); out[i * 6 + 4] = __fmaf_rn(a3, l4, __fmul_rn(a2, l1)); out[i * 6 + 5] = Lf[i * 6 + 5];
+    const float a[4] = {A[i * 4], A[i * 4 + 1], A[i * 4 + 2], A[i * 4 + 3]};
+    const float l[6] = {Lf[i * 6], Lf[i * 6 + 1], Lf[i * 6 + 2], Lf[i * 6 + 3], Lf[i * 6 + 4], Lf[i * 6 + 5]};
+    float o[6];
+    laf_left_mul(a, l, o);
+#pragma unroll
+    for (int q = 0; q < 6; q++) out[i * 6 + q] = o[q];
 }
 }  // namespace ag
 

@@ -26,22 +26,6 @@ __global__ void extract_patches_kernel(const float* __restrict__ img, int C, int
         out[((size_t)pi * C + c) * PS * PS + t] = bilinear_zero(base + (size_t)c * h * w, h, w, px, py);
 }
 
-struct PyrGeom {
-    int n_octaves, n_levels, B;
-    int h[AG_MAX_OCTAVES], w[AG_MAX_OCTAVES];
-    long long off[AG_MAX_OCTAVES][AG_MAX_LEVELS];
-};
-
-static PyrGeom make_geom(const ag_pyramid_plan_t* p) {
-    PyrGeom g;
-    g.n_octaves = p->n_octaves; g.n_levels = p->n_levels; g.B = p->B;
-    for (int o = 0; o < AG_MAX_OCTAVES; o++) {
-        g.h[o] = p->h[o]; g.w[o] = p->w[o];
-        for (int l = 0; l < AG_MAX_LEVELS; l++) g.off[o][l] = p->level_offset[o][l];
-    }
-    return g;
-}
-
 __global__ void extract_patches_pyr_kernel(const PyrGeom G, const float* __restrict__ pyr, const float* __restrict__ lafs,
                                            const int* __restrict__ oct, const int* __restrict__ lvl,
                                            const int* __restrict__ count, int cap, int PS, float* __restrict__ out) {

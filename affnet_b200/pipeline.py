@@ -6,14 +6,47 @@ import ctypes as C
 import torch
 
 from . import _lib as L
+from ._nets import _NativeNet
+from .HandCraftedModules import AffineShapeEstimator, OrientationDetector
+
+
+def _estimators(AffNet, OriNet, num_Baum_iters, do_ori):
+    """The estimator modes of ScaleSpaceAffinePatchExtractor's constructor, chosen by module type: AffNet is an AffNetFast or an
+    AffineShapeEstimator (may be None with num_Baum_iters=0); OriNet an OriNetFast or an OrientationDetector.  A missing net is left
+    to the library, which refuses the combination with its message."""
+    n = int(num_Baum_iters)
+    if isinstance(AffNet, AffineShapeEstimator):
+        shape, shape_ps = L.SHAPE_BAUMBERG, int(AffNet.PS)
+    elif AffNet is None or (isinstance(AffNet, _NativeNet) and AffNet.KIND == L.NET_AFFNET):
+        shape, shape_ps = L.SHAPE_AFFNET, 32
+    else:
+        raise L.AffnetB200Error("AffNet must be an AffNetFast, an AffineShapeEstimator or None, not %s" % type(AffNet).__name__)
+    if not do_ori:
+        ori, ori_ps = L.ORI_NONE, 0
+    elif isinstance(OriNet, OrientationDetector):
+        ori, ori_ps = L.ORI_HIST, int(OriNet.PS)
+    elif OriNet is None or (isinstance(OriNet, _NativeNet) and OriNet.KIND == L.NET_ORINET):
+        ori, ori_ps = L.ORI_ORINET, 32
+    else:
+        raise L.AffnetB200Error("OriNet must be an OriNetFast or an OrientationDetector, not %s" % type(OriNet).__name__)
+    return L.PipelineEstimators(shape, n, shape_ps, ori, ori_ps)
+
+
+def _handle(m):
+    """ag_net_t of a CNN module; the hand-crafted estimators have none (the library derives their windows from the patch size)."""
+    return m.handle() if isinstance(m, _NativeNet) else None
 
 
 class DetectDescribePipeline:
     def __init__(self, B, H, W, AffNet, HardNet, OriNet=None, num_features=2000, border=5, mrSize=5.192, nlevels=3,
-                 init_sigma=1.6, do_ori=True, cand_cap=0, device="cuda", outputs=None):
+                 init_sigma=1.6, do_ori=True, cand_cap=0, device="cuda", outputs=None, num_Baum_iters=1):
         """outputs: optional list of (lafs [B,K,2,3], desc [B,K,128], count [B] int32) CUDA tensors, one tuple per output slot, that the
-        kernels write into directly (e.g. DescriptorExchange.outputs(): the blocks an all-gather sends); default: one private slot."""
+        kernels write into directly (e.g. DescriptorExchange.outputs(): the blocks an all-gather sends); default: one private slot.
+        Estimators as ScaleSpaceAffinePatchExtractor selects them: AffNet = AffNetFast (num_Baum_iters AffNet iterations) or
+        AffineShapeEstimator (num_Baum_iters Baumberg iterations), either or None with num_Baum_iters=0 (no shape stage); with do_ori,
+        OriNet = OriNetFast or OrientationDetector (gradient histogram).  Patch sizes come from the modules."""
         self.cfg = L.PipelineConfig(B, H, W, num_features, nlevels, border, float(init_sigma), float(mrSize), 1 if do_ori else 0, cand_cap)
+        self.est = _estimators(AffNet, OriNet, num_Baum_iters, do_ori)
         self.nets = (AffNet, OriNet, HardNet)  # keep the modules alive; the C pipeline only BORROWS their ag_net_t handles
         self._h = None
         self._net_handles = None
@@ -42,16 +75,16 @@ class DetectDescribePipeline:
         the handle objects it was built with against the modules' and rebinds (run) or refuses (replay: the captured graph holds the
         old weight pointers) when they differ."""
         AffNet, OriNet, HardNet = self.nets
-        hs = (AffNet.handle(), OriNet.handle() if OriNet is not None else None, HardNet.handle())
+        hs = (_handle(AffNet), _handle(OriNet), _handle(HardNet))
         if self._h is not None:
             L.lib().ag_pipeline_destroy(self._h)
             self._h = None
         h = C.c_void_p()
-        L.check(L.lib().ag_pipeline_create(C.byref(self.cfg), hs[0], hs[1], hs[2], C.byref(h)))
+        L.check(L.lib().ag_pipeline_create_ex(C.byref(self.cfg), C.byref(self.est), hs[0], hs[1], hs[2], C.byref(h)))
         self._h, self._net_handles, self._graph = h, hs, None
 
     def _nets_current(self):
-        return all(n is None or n._handle is h for n, h in zip(self.nets, self._net_handles))
+        return all(not isinstance(n, _NativeNet) or n._handle is h for n, h in zip(self.nets, self._net_handles))
 
     def __del__(self):
         try:
@@ -67,7 +100,7 @@ class DetectDescribePipeline:
         """imgs CUDA float32 [B,1,H,W] or [B,H,W] -> (lafs [B,K,2,3] px, resp [B,K], desc [B,K,128], count [B]) of output slot `slot`.
         Rows >= count[b] are unspecified.  No host synchronisation."""
         imgs = L.f32c(imgs, "imgs")
-        if not self._nets_current() or any(n is not None and n.handle() is not h for n, h in zip(self.nets, self._net_handles)):
+        if not self._nets_current() or any(isinstance(n, _NativeNet) and n.handle() is not h for n, h in zip(self.nets, self._net_handles)):
             self._bind_nets()      # a net was reloaded / moved since the pipeline was built
         if imgs.numel() != self.B * self.H * self.W:
             raise L.AffnetB200Error("expected %d x %d x %d pixels" % (self.B, self.H, self.W))

@@ -251,6 +251,19 @@ int ag_lafs_to_ell(const float* d_lafs, int n, float* d_ell, void* stream);
 int ag_circular_gauss_kernel(int kernlen, double sigma, float* h_out);
 int ag_orientation_hist(const float* d_patches, int n, int PS, const float* d_gk, float* d_angle, void* stream);
 int ag_baumberg_shape(const float* d_patches, int n, int PS, const float* d_gk, float* d_A, void* stream);
+/* The same estimators sampling their patches from the pyramid inside the kernel (PS x PS patches never reach HBM).  Layout as
+ * ag_extract_patches_pyr: d_lafs [B,cap,2,3] normalised, d_oct/d_lvl [B,cap], d_count [B] (NULL => all rows); rows i >= d_count[b] are
+ * neither read nor written.  The Gaussian window is derived from PS as the modules derive it.  3 <= PS <= 41.
+ *   ag_orientation_hist_pyr = ag_extract_patches_pyr -> ag_orientation_hist -> (cos, sin) -> ag_lafs_apply_rotation, bit for bit:
+ *                             d_angle [B,cap] and/or d_lafs_out [B,cap,2,3] = [LAF_A * R | t], R = [[c, s], [-s, c]]; either may be
+ *                             NULL (not both); d_lafs_out may equal d_lafs (rotates in place).
+ *   ag_baumberg_shape_pyr   = the n_iters loop of getAffineShape (SparseImgRepresenter.py:155-166) over ag_extract_patches_pyr ->
+ *                             ag_baumberg_shape -> ag_mat2_compose -> ag_lafs_left_multiply, bit for bit, in one launch:
+ *                             d_A [B,cap,2,2] = base_A (1 <= n_iters <= 64). */
+int ag_orientation_hist_pyr(const ag_pyramid_plan_t* plan, const float* d_pyr, const float* d_lafs, const int* d_oct,
+                            const int* d_lvl, const int* d_count, int cap, int PS, float* d_angle, float* d_lafs_out, void* stream);
+int ag_baumberg_shape_pyr(const ag_pyramid_plan_t* plan, const float* d_pyr, const float* d_lafs, const int* d_oct,
+                          const int* d_lvl, const int* d_count, int cap, int PS, int n_iters, float* d_A, void* stream);
 
 /* Descriptor matching (SURVEY.md §8f row 3).
  *   ag_distance_matrix replaces distance_matrix_vector (Losses.py:5-13): out[n1,n2] = sqrt(|a|^2 + |b|^2 - 2 a.b + 1e-6)
@@ -266,6 +279,8 @@ int ag_match_snn(const float* d_desc1, int n1, const float* d_desc2, int n2, int
  * Batched end-to-end pipeline (new; the reference processes one image at a time):
  * pyramid -> detect -> select(1.5K) -> sample -> AffNet -> filter(K) -> [sample -> OriNet -> rotate]
  * -> denormalise -> level select -> sample -> HardNet.       = ScaleSpaceAffinePatchExtractor.forward
+ * (the default estimators; ag_pipeline_create_ex selects the others: AffNet or Baumberg x num_Baum_iters or no shape
+ * stage, OriNet, histogram or no orientation)
  * + extract_patches_from_pyr + HardNet.forward (train_AffNet_test_on_graffity.py:255-260) for B images.
  * ------------------------------------------------------------------------------------------ */
 typedef struct ag_pipeline ag_pipeline_t;
@@ -282,9 +297,36 @@ typedef struct {
 } ag_pipeline_config_t;
 
 /* Nets are borrowed (must outlive the pipeline).  The pipeline owns no device memory: the caller passes one
- * workspace of ag_pipeline_workspace_bytes() bytes. */
+ * workspace of ag_pipeline_workspace_bytes() bytes.  Same as ag_pipeline_create_ex(cfg, NULL, ...). */
 int ag_pipeline_create(const ag_pipeline_config_t* cfg, const ag_net_t* affnet, const ag_net_t* orinet,
                        const ag_net_t* hardnet, ag_pipeline_t** out);
+
+/* Estimator configuration of the pipeline: the choices of ScaleSpaceAffinePatchExtractor's constructor
+ * (SparseImgRepresenter.py:14-49) for the affine shape and orientation stages.
+ *   shape          AG_SHAPE_AFFNET: num_Baum_iters AffNet iterations (sampler fused into the net), needs `affnet`;
+ *                  AG_SHAPE_BAUMBERG: num_Baum_iters Baumberg iterations (AffineShapeEstimator) in one ag_baumberg_shape_pyr launch.
+ *   num_Baum_iters 0..64; 0 = no shape stage: the K strongest keypoints go straight from the detector to orientation.
+ *                  With 1 or more iterations int(1.5 K) keypoints are selected and the shape filter keeps K.
+ *   shape_ps       patch size of the Baumberg estimator (3..41; 19 in the reference); ignored for AffNet (32).
+ *   ori            AG_ORI_NONE; AG_ORI_ORINET (needs `orinet`); AG_ORI_HIST: gradient-histogram OrientationDetector,
+ *                  one ag_orientation_hist_pyr launch.
+ *   ori_ps         patch size of the histogram orientation (3..41; 19 in the reference); ignored otherwise.
+ * est == NULL gives AG_SHAPE_AFFNET with 1 iteration and cfg->do_ori ? AG_ORI_ORINET : AG_ORI_NONE (ag_pipeline_create).
+ * With est != NULL, est->ori governs and cfg->do_ori is ignored.  Invalid combinations fail here with AG_ERR_INVALID. */
+#define AG_SHAPE_AFFNET 0
+#define AG_SHAPE_BAUMBERG 1
+#define AG_ORI_NONE 0
+#define AG_ORI_ORINET 1
+#define AG_ORI_HIST 2
+typedef struct {
+    int shape;           /* AG_SHAPE_* */
+    int num_Baum_iters;  /* 0..64 */
+    int shape_ps;        /* Baumberg patch size */
+    int ori;             /* AG_ORI_* */
+    int ori_ps;          /* histogram-orientation patch size */
+} ag_pipeline_estimators_t;
+int ag_pipeline_create_ex(const ag_pipeline_config_t* cfg, const ag_pipeline_estimators_t* est, const ag_net_t* affnet,
+                          const ag_net_t* orinet, const ag_net_t* hardnet, ag_pipeline_t** out);
 void ag_pipeline_destroy(ag_pipeline_t* p);
 size_t ag_pipeline_workspace_bytes(const ag_pipeline_t* p);
 const ag_pyramid_plan_t* ag_pipeline_plan(const ag_pipeline_t* p);
