@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("AFFNET_B200_LIB", os.path.join(HERE, "lib", "libaffnet_b200.so"))   # override: developer builds only
 AG_MAX_OCTAVES, AG_MAX_LEVELS = 16, 8
 NET_AFFNET, NET_ORINET, NET_HARDNET = 0, 1, 2
-ENGINE_SIMT, ENGINE_TC, ENGINE_TC_EXACT, ENGINE_TC_FAST, ENGINE_TC2, ENGINE_TC2_BF16 = 0, 1, 2, 3, 4, 5
+ENGINE_SIMT, ENGINE_TC2, ENGINE_TC2_BF16 = 0, 4, 5
 
 
 class AffnetB200Error(RuntimeError):
@@ -87,7 +87,6 @@ PROTOTYPES = {
     "ag_lafs_left_multiply": (i32, [vp, vp, vp, i32, vp]),
     "ag_affnet_forward_raw": (i32, [vp, vp, i32, vp, vp, sz, vp]),
     "ag_orinet_forward_raw": (i32, [vp, vp, i32, vp, vp, sz, vp]),
-    "ag_debug_pyramid_mode": (i32, [i32]),
     "ag_debug_fuse_l3": (i32, [i32]),
     "ag_debug_tcx_layer": (i32, [vp, vp, i32, i32, vp, vp, sz, vp]),
     "ag_affnet_forward": (i32, [vp, vp, i32, vp, i32, vp, vp, sz, vp]),

@@ -60,12 +60,11 @@ class _NativeNet(nn.Module):
         return self._handle
 
     def set_engine(self, engine):
-        """engine: L.ENGINE_TC2 (second-generation tcgen05 engine, default), L.ENGINE_TC2_BF16 (HardNet with bf16 operands), L.ENGINE_SIMT
-        (exact fp32 CUDA cores), L.ENGINE_TC / L.ENGINE_TC_EXACT / L.ENGINE_TC_FAST (first-generation tcgen05 engine and its variants); see
-        include/affnet_b200.h."""
-        self._engine = engine
+        """engine: L.ENGINE_TC2 (tcgen05 tensor-core engine, default), L.ENGINE_TC2_BF16 (HardNet with bf16 operands) or L.ENGINE_SIMT
+        (exact fp32 CUDA cores); see include/affnet_b200.h.  Any other value raises AffnetB200Error once the net has a handle."""
         if self._handle is not None:
             L.check(L.lib().ag_net_set_engine(self._handle, engine))
+        self._engine = engine
         return self
 
     @property

@@ -238,197 +238,26 @@ __global__ void __launch_bounds__(DNT) detect_level_kernel(const DetectParams P)
 
 
 // ======================================================================================================================
-// Fused single-launch detector for nlevels = 3 (the reference's only configuration): one CTA stages a 36x36 window of all
-// FIVE pyramid levels of its octave, derives the five 34x34 response windows once, and runs the three detection levels
-// from shared memory.  The reference's sequential octave-map logic (level k sees the map left by the accepted levels
-// below it; a level with <= 1 positive maxima is dropped and leaves no trace, HandCraftedModules.py:246-256) is made
-// launch-free by counting every acceptance hypothesis (a1, a2 in {0,1}) in the same pass and storing, with each candidate,
-// the raw NMS values of the same pixel at the levels below; `resolve_kernel` then picks the branch the counters select and
-// computes the masked response with the reference's exact fp32 / uint8-wrap arithmetic.
+// Single-launch detector for nlevels = 3 (the reference's only configuration): each pass reads all FIVE pyramid levels of its
+// octave, derives the five response maps once, and runs the three detection levels together.  The reference's sequential
+// octave-map logic (level k sees the map left by the accepted levels below it; a level with <= 1 positive maxima is dropped and
+// leaves no trace, HandCraftedModules.py:246-256) is made launch-free by counting every acceptance hypothesis (a1, a2 in {0,1}) in
+// the same pass and storing, with each candidate, the raw NMS values of the same pixel at the levels below; `resolve_kernel` then
+// picks the branch the counters select and computes the masked response with the reference's exact fp32 / uint8-wrap arithmetic.
 // ======================================================================================================================
 constexpr int NVAR = 16;  // per (image, octave): [0] pos1, [1..2] pos2[a1], [3..6] pos3[a1][a2], [7] emit1, [8..9] emit2[a1], [10..13] emit3[a1][a2]
-
-struct FusedOctave {
-    const float* lvl[5];
-    float s4[5], sc[5];
-    int h, w, tiles_x, tiles_y, tile_base;
-};
-struct FusedParams {
-    FusedOctave oct[AG_MAX_OCTAVES];
-    int n_oct, total_tiles;
-    float th;
-    int mr_border, cand_cap;
-    float* cand_val;
-    float* cand_aux;
-    uint32_t* cand_seq;
-    float* cand_scyx;
-    int* cand_count;
-    int* variants;  // [B][n_oct][NVAR]
-};
 
 __device__ __forceinline__ uint8_t om_after(uint8_t om, float val) { return float_to_u8_wrap(__fadd_rn((float)om, val)); }
 __device__ __forceinline__ float masked(float nms, uint8_t om) { return __fmul_rn(nms, __fsub_rn(1.0f, (float)om)); }
 
-__global__ void __launch_bounds__(DNT) detect_fused_kernel(const FusedParams P) {
-    extern __shared__ __align__(16) float s_dyn[];
-    float (*s_a)[PW][PW + 1] = reinterpret_cast<float (*)[PW][PW + 1]>(s_dyn);                            // pyramid windows, later row-max maps
-    float (*s_resp)[RW][RW + 1] = reinterpret_cast<float (*)[RW][RW + 1]>(s_dyn + 5 * PW * (PW + 1));     // response windows
-    __shared__ int s_var[NVAR];
-    __shared__ int s_base[2];
-    int t = blockIdx.x, oi = 0;
-#pragma unroll 1
-    for (int i = 1; i < P.n_oct; i++)
-        if (t >= P.oct[i].tile_base) oi = i;
-    const FusedOctave& O = P.oct[oi];
-    t -= O.tile_base;
-    const int b = blockIdx.y, h = O.h, w = O.w;
-    const int ty = t / O.tiles_x, tx = t - ty * O.tiles_x;
-    const int y0 = ty * DT, x0 = tx * DT;
-    const size_t img_off = (size_t)b * h * w;
-    if (threadIdx.x < NVAR) s_var[threadIdx.x] = 0;
-    if (threadIdx.x < 2) s_base[threadIdx.x] = 0;
-    // 1. pyramid windows (origin y0-2, x0-2), replicate-clamped
-#pragma unroll
-    for (int d = 0; d < 5; d++) {
-        const float* src = O.lvl[d] + img_off;
-        for (int i = threadIdx.x; i < PW * PW; i += DNT) {
-            const int ly = i / PW, lx = i - ly * PW;
-            s_a[d][ly][lx] = __ldg(src + (size_t)clampi(y0 - 2 + ly, 0, h - 1) * w + clampi(x0 - 2 + lx, 0, w - 1));
-        }
-    }
-    __syncthreads();
-    // 2. response windows (origin y0-1, x0-1), zero outside the image
-#pragma unroll
-    for (int d = 0; d < 5; d++)
-        for (int i = threadIdx.x; i < RW * RW; i += DNT) {
-            const int ly = i / RW, lx = i - ly * RW;
-            const int gy = y0 - 1 + ly, gx = x0 - 1 + lx;
-            s_resp[d][ly][lx] = (gy >= 0 && gy < h && gx >= 0 && gx < w) ? hessian_at(s_a[d], ly + 1, lx + 1, O.s4[d], P.th) : 0.f;
-        }
-    __syncthreads();
-    // 3. separable 3x3 max: row pass into the (dead) pyramid windows.  Zero padding is exact: responses are >= 0 and the
-    //    centre always takes part in the max.
-    float (*s_rm)[RW][DT] = reinterpret_cast<float (*)[RW][DT]>(&s_a[0][0][0]);
-    for (int i = threadIdx.x; i < 5 * RW * DT; i += DNT) {
-        const int d = i / (RW * DT), r = i - d * RW * DT, ly = r / DT, j = r - ly * DT;
-        s_rm[d][ly][j] = fmaxf(fmaxf(s_resp[d][ly][j], s_resp[d][ly][j + 1]), s_resp[d][ly][j + 2]);
-    }
-    __syncthreads();
-    // 4. per pixel: three NMS decisions, hypothesis counters, candidate slots
-    const bool border_ok = (P.mr_border < w) && (P.mr_border < h);
-    constexpr int PPT = DT * DT / DNT;
-    float nms[PPT][3];
-    int var[NVAR];
-#pragma unroll
-    for (int i = 0; i < NVAR; i++) var[i] = 0;
-    int n_emit = 0;
-#pragma unroll
-    for (int k = 0; k < PPT; k++) {
-        const int i = threadIdx.x + k * DNT, ly = i / DT, lx = i - ly * DT;
-        const int gy = y0 + ly, gx = x0 + lx;
-        nms[k][0] = nms[k][1] = nms[k][2] = 0.f;
-        if (gy < h && gx < w && border_ok && gy >= P.mr_border && gy < h - P.mr_border && gx >= P.mr_border && gx < w - P.mr_border) {
-            float M[5];
-#pragma unroll
-            for (int d = 0; d < 5; d++) M[d] = fmaxf(fmaxf(s_rm[d][ly][lx], s_rm[d][ly + 1][lx]), s_rm[d][ly + 2][lx]);
-#pragma unroll
-            for (int q = 0; q < 3; q++) {
-                const float x = s_resp[q + 1][ly + 1][lx + 1];
-                const float m = fmaxf(fmaxf(M[q], M[q + 1]), M[q + 2]);
-                nms[k][q] = (__fadd_rn(__fsub_rn(x, m), 1e-5f) > 0.f) ? x : 0.f;   // NMS3d, HandCraftedModules.py:220
-            }
-            const float n1 = nms[k][0], n2 = nms[k][1], n3 = nms[k][2];
-            if (n1 != 0.f || n2 != 0.f || n3 != 0.f) {
-                n_emit += (n1 != 0.f) + (n2 != 0.f) + (n3 != 0.f);
-                var[0] += n1 > 0.f; var[7] += n1 != 0.f;
-#pragma unroll
-                for (int a1 = 0; a1 < 2; a1++) {
-                    const uint8_t om1 = a1 ? om_after(0, n1) : (uint8_t)0;
-                    const float v2 = masked(n2, om1);
-                    var[1 + a1] += v2 > 0.f; var[8 + a1] += v2 != 0.f;
-#pragma unroll
-                    for (int a2 = 0; a2 < 2; a2++) {
-                        const uint8_t om2 = a2 ? om_after(om1, v2) : om1;
-                        const float v3 = masked(n3, om2);
-                        var[3 + a1 * 2 + a2] += v3 > 0.f; var[10 + a1 * 2 + a2] += v3 != 0.f;
-                    }
-                }
-            }
-        }
-    }
-    const unsigned lane = threadIdx.x & 31;
-    const unsigned any = __ballot_sync(0xffffffffu, n_emit > 0);
-    int incl = n_emit, warp_base = 0;
-    if (any) {
-#pragma unroll
-        for (int i = 0; i < 14; i++) {
-            int v = var[i];
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-            if (lane == 0 && v) atomicAdd(&s_var[i], v);
-        }
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int v = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= (unsigned)o) incl += v;
-        }
-        const int wsum = __shfl_sync(0xffffffffu, incl, 31);
-        if (lane == 0) warp_base = atomicAdd(&s_base[0], wsum);
-        warp_base = __shfl_sync(0xffffffffu, warp_base, 0);
-    }
-    __syncthreads();
-    if (s_base[0] == 0) return;
-    if (threadIdx.x < 14 && s_var[threadIdx.x]) atomicAdd(&P.variants[((size_t)b * P.n_oct + oi) * NVAR + threadIdx.x], s_var[threadIdx.x]);
-    if (threadIdx.x == 0) s_base[1] = atomicAdd(&P.cand_count[b], s_base[0]);
-    __syncthreads();
-    if (n_emit == 0) return;
-    int dst = s_base[1] + warp_base + (incl - n_emit);
-    // 5. soft-argmax + emission (HandCraftedModules.py:266-290)
-    const float min_size = (float)min(h, w);
-#pragma unroll
-    for (int k = 0; k < PPT; k++) {
-        const int i = threadIdx.x + k * DNT, ly = i / DT, lx = i - ly * DT;
-        const int gy = y0 + ly, gx = x0 + lx;
-#pragma unroll
-        for (int q = 0; q < 3; q++) {
-            if (nms[k][q] == 0.f) continue;
-            if (dst < P.cand_cap) {
-                float ns = 0.f, ny = 0.f, nx = 0.f, den = 0.f;
-#pragma unroll
-                for (int d = 0; d < 3; d++)
-#pragma unroll
-                    for (int dy = 0; dy < 3; dy++)
-#pragma unroll
-                        for (int dx = 0; dx < 3; dx++) {
-                            const float r = s_resp[q + d][ly + dy][lx + dx];
-                            ns = fmaf(O.sc[q + d], r, ns);
-                            ny = fmaf(-0.5f + (float)dy, r, ny);
-                            nx = fmaf(-0.5f + (float)dx, r, nx);
-                            den += r;
-                        }
-                den = __fadd_rn(den, 1e-8f);
-                const size_t o = (size_t)b * P.cand_cap + dst;
-                P.cand_val[o] = nms[k][q];
-                P.cand_aux[o * 2 + 0] = nms[k][0];
-                P.cand_aux[o * 2 + 1] = nms[k][1];
-                P.cand_seq[o] = ((uint32_t)(oi * 3 + q) << SEQ_PIX_BITS) | (uint32_t)(gy * w + gx);
-                P.cand_scyx[o * 3 + 0] = __fdiv_rn(__fdiv_rn(ns, den), min_size);
-                P.cand_scyx[o * 3 + 1] = __fdiv_rn(__fadd_rn(__fdiv_rn(ny, den), (float)gy), (float)h);
-                P.cand_scyx[o * 3 + 2] = __fdiv_rn(__fadd_rn(__fdiv_rn(nx, den), (float)gx), (float)w);
-            }
-            dst++;
-        }
-    }
-}
-
 
 // ======================================================================================================================
-// Register-resident formulation of the fused detector: one warp owns a band of rows of a 30-column strip (32 lanes = 30
+// Register-resident formulation of the single-launch detector: one warp owns a band of rows of a 30-column strip (32 lanes = 30
 // output columns + one response-halo column each side), walks down the rows keeping three pyramid rows of all five levels
 // in registers, takes horizontal neighbours by warp shuffle, and never touches shared memory on the common path:
 //   per pixel and level: 1 coalesced load + 2 shuffles + the Hessian; separable 3x3 max via 2 shuffles + FMNMX3.
 // Candidates (about 1 % of the pixels) take a warp-cooperative slow path that gathers the 3x3x3 response neighbourhood by
-// shuffle for the soft-argmax.  Semantics are identical to detect_fused_kernel (same hypothesis counters, same records).
+// shuffle for the soft-argmax.
 // ======================================================================================================================
 constexpr int WCOLS = 30;   // output columns per warp strip
 #ifndef AG_WROWS
@@ -667,7 +496,7 @@ __global__ void __launch_bounds__(WNT) detect_warp_kernel(const WarpParams P) {
 //   * the row loop is unrolled by three with compile-time slot indices: no register rotation;
 //   * the row fetch is branch-free: one cp.async per level from a per-lane offset, the two halo columns by a predicated second one;
 //   * the soft-argmax divisions move to the candidate flush, where 32 lanes finish 32 candidates at once.
-// Records, counters and their semantics are those of detect_warp_kernel / detect_fused_kernel.
+// Records, counters and their semantics are those of detect_warp_kernel.
 // ======================================================================================================================
 template <int I> struct IC { static constexpr int value = I; };
 
@@ -1200,68 +1029,41 @@ int ag_detect(const ag_pyramid_plan_t* p, const float* d_pyr, float th, int mr_b
                         "memset counters");
     if (rc != AG_OK) return rc;
     if (n_det == 3) {
-        // single-launch fused detector + hypothesis resolution
-        FusedParams F;
-        memset(&F, 0, sizeof(F));
-        F.n_oct = p->n_octaves; F.th = th; F.mr_border = mr_border; F.cand_cap = ws->cand_cap;
-        F.cand_val = ws->d_cand_val; F.cand_aux = ws->d_cand_aux; F.cand_seq = ws->d_cand_seq; F.cand_scyx = ws->d_cand_scyx;
-        F.cand_count = ws->d_cand_count; F.variants = ws->d_variants;
-        int tiles = 0;
+        // single-launch detector + hypothesis resolution
+        WarpParams Wp;
+        memset(&Wp, 0, sizeof(Wp));
+        Wp.n_oct = p->n_octaves; Wp.th = th; Wp.mr_border = mr_border; Wp.cand_cap = ws->cand_cap;
+        Wp.cand_val = ws->d_cand_val; Wp.cand_aux = ws->d_cand_aux; Wp.cand_seq = ws->d_cand_seq; Wp.cand_scyx = ws->d_cand_scyx;
+        Wp.cand_count = ws->d_cand_count; Wp.variants = ws->d_variants;
+        int units = 0;
         for (int o = 0; o < p->n_octaves; o++) {
-            FusedOctave& O = F.oct[o];
+            WarpOctave& O = Wp.oct[o];
             for (int d = 0; d < 5; d++) {
                 O.lvl[d] = d_pyr + p->level_offset[o][d];
                 O.s4[d] = (float)pow(p->sigma[o][d], 4.0);
                 O.sc[d] = (float)p->sigma[o][d];
             }
             O.h = p->h[o]; O.w = p->w[o];
-            O.tiles_x = cdiv(O.w, DT); O.tiles_y = cdiv(O.h, DT);
-            O.tile_base = tiles;
-            tiles += O.tiles_x * O.tiles_y;
+            O.strips_x = cdiv(O.w, WCOLS); O.bands_y = cdiv(O.h, WROWS);
+            O.unit_base = units;
+            units += O.strips_x * O.bands_y;
         }
-        F.total_tiles = tiles;
-        static const bool use_tiled = getenv("AG_DETECT_TILED") != nullptr;   // A/B switch: shared-memory tiled variant
-        if (!use_tiled) {
-            WarpParams Wp;
-            memset(&Wp, 0, sizeof(Wp));
-            Wp.n_oct = p->n_octaves; Wp.th = th; Wp.mr_border = mr_border; Wp.cand_cap = ws->cand_cap;
-            Wp.cand_val = ws->d_cand_val; Wp.cand_aux = ws->d_cand_aux; Wp.cand_seq = ws->d_cand_seq; Wp.cand_scyx = ws->d_cand_scyx;
-            Wp.cand_count = ws->d_cand_count; Wp.variants = ws->d_variants;
-            int units = 0;
-            for (int o = 0; o < p->n_octaves; o++) {
-                WarpOctave& O = Wp.oct[o];
-                for (int d = 0; d < 5; d++) { O.lvl[d] = F.oct[o].lvl[d]; O.s4[d] = F.oct[o].s4[d]; O.sc[d] = F.oct[o].sc[d]; }
-                O.h = p->h[o]; O.w = p->w[o];
-                O.strips_x = cdiv(O.w, WCOLS); O.bands_y = cdiv(O.h, WROWS);
-                O.unit_base = units;
-                units += O.strips_x * O.bands_y;
-            }
-            Wp.total_units = units;
-            static const bool use_v1 = getenv("AG_DETECT_WARP_V1") != nullptr;     // A/B switch: the first register formulation
-            // detect_rows_kernel addresses an octave's levels with 32-bit element offsets from its first level
-            bool fits32 = true;
-            for (int o = 0; o < p->n_octaves; o++) {
-                long long lo = 0, hi = 0;
-                for (int d = 0; d < 5; d++) { const long long off = Wp.oct[o].lvl[d] - Wp.oct[o].lvl[0]; lo = off < lo ? off : lo; hi = off > hi ? off : hi; }
-                if (lo < -(1ll << 30) || hi + (long long)p->B * p->h[o] * p->w[o] >= (1ll << 31) - 64) fits32 = false;
-            }
-            if (use_v1 || !fits32) {
-                detect_warp_kernel<<<dim3(cdiv(units, WNT / 32), p->B), WNT, 0, st>>>(Wp);
-                AG_CHECK_LAUNCH("detect_warp_kernel");
-            } else {
-                detect_rows_kernel<<<dim3(cdiv(units, WNT / 32), p->B), WNT, 0, st>>>(Wp);
-                AG_CHECK_LAUNCH("detect_rows_kernel");
-            }
-            resolve_kernel<<<dim3(8, p->B), 256, 0, st>>>(ws->d_variants, p->n_octaves, ws->cand_cap, ws->d_cand_count, ws->d_cand_val, ws->d_cand_aux,
-                                                           ws->d_cand_seq, ws->d_level_pos, ws->d_level_emit);
-            AG_CHECK_LAUNCH("resolve_kernel");
-            return AG_OK;
+        Wp.total_units = units;
+        static const bool use_v1 = getenv("AG_DETECT_WARP_V1") != nullptr;     // A/B switch: the first register formulation
+        // detect_rows_kernel addresses an octave's levels with 32-bit element offsets from its first level
+        bool fits32 = true;
+        for (int o = 0; o < p->n_octaves; o++) {
+            long long lo = 0, hi = 0;
+            for (int d = 0; d < 5; d++) { const long long off = Wp.oct[o].lvl[d] - Wp.oct[o].lvl[0]; lo = off < lo ? off : lo; hi = off > hi ? off : hi; }
+            if (lo < -(1ll << 30) || hi + (long long)p->B * p->h[o] * p->w[o] >= (1ll << 31) - 64) fits32 = false;
         }
-        constexpr size_t fsmem = sizeof(float) * (5 * PW * (PW + 1) + 5 * RW * (RW + 1));
-        static SmemAttrOnce attr_once;
-        if ((rc = attr_once.ensure(detect_fused_kernel, fsmem, "detect smem attr")) != AG_OK) return rc;
-        detect_fused_kernel<<<dim3(tiles, p->B), DNT, fsmem, st>>>(F);
-        AG_CHECK_LAUNCH("detect_fused_kernel");
+        if (use_v1 || !fits32) {
+            detect_warp_kernel<<<dim3(cdiv(units, WNT / 32), p->B), WNT, 0, st>>>(Wp);
+            AG_CHECK_LAUNCH("detect_warp_kernel");
+        } else {
+            detect_rows_kernel<<<dim3(cdiv(units, WNT / 32), p->B), WNT, 0, st>>>(Wp);
+            AG_CHECK_LAUNCH("detect_rows_kernel");
+        }
         resolve_kernel<<<dim3(8, p->B), 256, 0, st>>>(ws->d_variants, p->n_octaves, ws->cand_cap, ws->d_cand_count, ws->d_cand_val, ws->d_cand_aux,
                                                        ws->d_cand_seq, ws->d_level_pos, ws->d_level_emit);
         AG_CHECK_LAUNCH("resolve_kernel");

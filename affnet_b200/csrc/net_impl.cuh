@@ -1,5 +1,5 @@
 // Internal definition of the opaque ag_net_t handle shared by the fp32 SIMT engine (nets_simt.cu) and the
-// tensor-core engine (nets_tc.cu).
+// tensor-core engine (nets_tcx.cu).
 #pragma once
 #include <cuda_fp16.h>
 
@@ -7,13 +7,11 @@
 
 #include "common.cuh"
 
-#define AG_ENGINE_SIMT 0  /* exact fp32 direct convolution */
-#define AG_ENGINE_TC 1    /* tcgen05: fp16 operands, fp32 accumulate in TMEM, heads as tensor-core GEMMs; AffNet / OriNet with fp16 residual planes of weights and activations (fp32-grade), HardNet plain fp16 */
-#define AG_ENGINE_TC_EXACT 2 /* tcgen05 trunk with fp16 residual planes of weights AND activations, heads as fp32 FMA chains */
-#define AG_ENGINE_TC2 4      /* second-generation tcgen05 engine (tcx_*.cuh): kernel-row taps stacked along N, same numerics contract as engine 1 plus
-                                HardNet weight residuals in layers 2-3 */
+#define AG_ENGINE_SIMT 0     /* exact fp32 direct convolution */
+#define AG_ENGINE_TC2 4      /* tcgen05 engine (tcx_*.cuh): fp16 operands, fp32 accumulate in TMEM, kernel-row taps stacked along N, heads as tensor-core
+                                GEMMs; AffNet / OriNet with fp16 residual planes of weights and activations (fp32-grade), HardNet with weight residuals
+                                in layers 2-3 */
 #define AG_ENGINE_TC2_BF16 5 /* HardNet only: engine 4 with bf16 operands (BASELINE.json configs[4]); descriptors ~4e-3 of the fp32 reference */
-#define AG_ENGINE_TC_FAST 3  /* AffNet only: weight residuals but single fp16 activations (A error 2e-4: too coarse for the 1e-3 LAF contract once OriNet amplifies it, kept for A/B timing) */
 
 struct ag_net {
     int kind;
@@ -25,33 +23,22 @@ struct ag_net {
     __half* d_all_x;
     __half* d_wx_bf[6];   // HardNet: the same packs in bf16 (engine 5); storage type is 16 bits either way
     __half* d_headh_bf;
-    __half* d_wh[6];   // fp16 [nsplit][hi|lo][9][cin/8][cout/nsplit][8] for layers 1..5 (index 0 unused; lo only for AffNet/OriNet)
     __half* d_headh;   // head for the tensor-core GEMM, k = (pixel*C/8 + c/8)*8 + c%8: HardNet fp16 [8192/8][128][8]; AffNet / OriNet [4096/8][32 hi | 32 lo][8]
     float* d_head_w;   // AffNet [3][4096], OriNet w_eff[4096][18] (per-position shifted copies), HardNet [8192][128]
     float* d_head_b;   // AffNet bias[3], OriNet bias[2], HardNet {scale[128], shift[128]}
-    float w_inv_scale[6];   // tensor-core layers: 1 / (power-of-two scale of d_wh[l]); [0] = layer 1 (scaled in the kernel)
+    float w_inv_scale[6];   // tensor-core layers: 1 / (power-of-two scale of d_wx[l]); [0] = layer 1 (scaled in the kernel)
     float head_inv_scale;   // AffNet / OriNet tensor-core head: 1 / (power-of-two scale of d_headh)
     float* d_all;      // fp32 allocation
     __half* d_all_h;   // fp16 allocation
 };
 
-#include "tc_conv.cuh"
+#include "tcgen05.cuh"
 
 namespace ag {
-size_t tc_act_bytes(int kind);
-int tc_nsplit(int kind, int layer);
-int tc_split_w(int kind);
 tc::FirstSrc tc_src_patches(const float* patches);
 tc::FirstSrc tc_src_pyramid(const ag_pyramid_plan_t* p, const float* pyr, const float* lafs, const int* oct, const int* lvl, int cap);
-int tc_hardnet_forward(const ag_net* net, const tc::FirstSrc& src, int n, int group, const int* count, void* bufA, void* bufB, void* headbuf,
-                       float* out, cudaStream_t st);
-int tc_trunk_orinet(const ag_net* net, const tc::FirstSrc& src, int n, int group, const int* count, void* bufA, void* bufB, void* feat,
-                    cudaStream_t st);
-int tc_trunk_affnet(const ag_net* net, const tc::FirstSrc& src, int n, int group, const int* count, void* bufA, void* bufB, void* feat,
-                    cudaStream_t st);
 int tc_headx_forward(const ag_net* net, const void* feat, int n, int group, const int* count, float* out, float* angle, cudaStream_t st, float* raw = nullptr);
 size_t tc_headx_bytes(int n);
-// second-generation engine (nets_tcx.cu)
 void tcx_pack_layer(const float* wf, int ci, int co, int stride, int nsplit, int sw, float scale, std::vector<__half>& out, int bf16 = 0);
 int tcx_nsplit(int kind, int layer);
 int tcx_split_w(int kind, int layer);

@@ -5,7 +5,7 @@
 // (affine=False, eps 1e-5, running stats; folded into the weights at upload) + ReLU, then the 8x8 head.
 // This is the exact-fp32 engine: every layer is a direct convolution with the whole (padded) input of one
 // patch staged in shared memory, activations in NCHW through L2-resident scratch.  The tensor-core engine
-// (nets_tc.cu) replaces the inner layers where present; first layer (K=9) and heads stay here.
+// (nets_tcx.cu) is the default; ag_net_create below packs the weights of both.
 #include <math.h>
 
 #include <vector>
@@ -379,32 +379,9 @@ int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out
         packed.insert(packed.end(), bias, bias + no);
         while (packed.size() % 4) packed.push_back(0.f);
     }
-    // fp16 packs for the tensor-core engine: [nsplit][9][cin/8][hi rows | lo rows][8], layers 1..5
-    std::vector<__half> packed_h;
-    size_t wh_off[6] = {0, 0, 0, 0, 0, 0};
-    float w_scale[6] = {1.f, 1.f, 1.f, 1.f, 1.f, 1.f};
-    w_scale[0] = pow2_scale(packed.data() + w_off[0], (size_t)9 * cfg[0].cout);
-    const int sw = tc_split_w(kind);
-    for (int l = 1; l < 6; l++) {
-        const int ci = cfg[l].cin, co = cfg[l].cout, ns = tc_nsplit(kind, l), nt = co / ns, kc = ci / 8;
-        const float* wf = packed.data() + w_off[l];  // [tap][ci][co]
-        w_scale[l] = pow2_scale(wf, (size_t)9 * ci * co);
-        wh_off[l] = packed_h.size();
-        packed_h.resize(packed_h.size() + (size_t)9 * ci * co * (1 + sw));
-        __half* dst = packed_h.data() + wh_off[l];
-        for (int sp = 0; sp < ns; sp++)
-            for (int tap = 0; tap < 9; tap++)
-                for (int g = 0; g < kc; g++)
-                    for (int part = 0; part <= sw; part++)
-                        for (int nn = 0; nn < nt; nn++)
-                            for (int e = 0; e < 8; e++) {
-                                const float v = w_scale[l] * wf[((size_t)tap * ci + g * 8 + e) * co + sp * nt + nn];
-                                const __half hi = __float2half_rn(v);
-                                const __half val = part == 0 ? hi : __float2half_rn(v - __half2float(hi));
-                                // [nsplit][9][kc][hi rows | lo rows][8]
-                                dst[(((((size_t)sp * 9 + tap) * kc + g) * (1 + sw) + part) * nt + nn) * 8 + e] = val;
-                            }
-    }
+    // power-of-two scales of the tensor-core weight packs, layers 1..6
+    float w_scale[6];
+    for (int l = 0; l < 6; l++) w_scale[l] = pow2_scale(packed.data() + w_off[l], (size_t)9 * cfg[l].cin * cfg[l].cout);
     // second-generation packs (tcx_pack_layer): kernel-row blocks with the three taps stacked along N
     std::vector<__half> packed_x;
     size_t wx_off[6] = {0, 0, 0, 0, 0, 0};
@@ -433,13 +410,12 @@ int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out
                         memcpy(&packed_bf[headbf_off + (((size_t)(pix * 16 + cg)) * 128 + o) * 8 + e], &bv, 2);
                     }
     }
-    size_t headh_off = 0;
+    // fp16 head packs for the tensor-core head GEMMs
+    std::vector<__half> packed_h;
     float head_scale = 1.0f;
     if (kind == AG_NET_HARDNET) {
-        while (packed_h.size() % 8) packed_h.push_back(__float2half_rn(0.f));
-        headh_off = packed_h.size();
-        packed_h.resize(packed_h.size() + (size_t)8192 * 128);
-        __half* dst = packed_h.data() + headh_off;
+        packed_h.resize((size_t)8192 * 128);
+        __half* dst = packed_h.data();
         const float* hw = packed.data() + hw_off;  // [k = c*64 + p][cout]
         for (int pix = 0; pix < 64; pix++)
             for (int cg = 0; cg < 16; cg++)
@@ -449,10 +425,8 @@ int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out
     }
     if (kind != AG_NET_HARDNET) {   // AffNet (3 outputs) / OriNet (18 shifted outputs): [4096/8][32 hi rows | 32 lo rows][8]
         const int no = (kind == AG_NET_AFFNET) ? 3 : 18;
-        while (packed_h.size() % 8) packed_h.push_back(__float2half_rn(0.f));
-        headh_off = packed_h.size();
-        packed_h.resize(packed_h.size() + (size_t)4096 * 64, __float2half_rn(0.f));
-        __half* dst = packed_h.data() + headh_off;
+        packed_h.resize((size_t)4096 * 64, __float2half_rn(0.f));
+        __half* dst = packed_h.data();
         const float* hw = packed.data() + hw_off;
         // the weights are stored times a power of two that brings the largest one near 2^13: their fp16 residuals then stay in
         // the normal range (a residual below 6e-5 would lose bits as a subnormal); the epilogue multiplies by 1/scale, exactly
@@ -472,7 +446,7 @@ int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out
     ag_net* net = new ag_net();
     memset(net, 0, sizeof(*net));
     net->kind = kind;
-    net->engine = AG_ENGINE_TC2;   // second-generation tensor-core engine (nets_tcx.cu); AG_ENGINE_TC selects the first generation
+    net->engine = AG_ENGINE_TC2;   // tensor-core engine (nets_tcx.cu)
     net->head_inv_scale = 1.0f / head_scale;
     for (int l = 0; l < 6; l++) net->w_inv_scale[l] = 1.0f / w_scale[l];
     {
@@ -480,8 +454,7 @@ int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out
         if (rch != AG_OK) { delete net; return rch; }
         rch = check_cuda(cudaMemcpy(net->d_all_h, packed_h.data(), packed_h.size() * sizeof(__half), cudaMemcpyHostToDevice), "upload fp16 weights");
         if (rch != AG_OK) { cudaFree(net->d_all_h); delete net; return rch; }
-        for (int l = 1; l < 6; l++) net->d_wh[l] = net->d_all_h + wh_off[l];
-        net->d_headh = net->d_all_h + headh_off;
+        net->d_headh = net->d_all_h;
         rch = check_cuda(cudaMalloc(&net->d_all_x, packed_x.size() * sizeof(__half)), "cudaMalloc fp16 weights (second generation)");
         if (rch == AG_OK) rch = check_cuda(cudaMemcpy(net->d_all_x, packed_x.data(), packed_x.size() * sizeof(__half), cudaMemcpyHostToDevice), "upload fp16 weights");
         if (rch != AG_OK) { cudaFree(net->d_all_h); cudaFree(net->d_all_x); delete net; return rch; }
@@ -519,10 +492,8 @@ void ag_net_destroy(ag_net_t* net) {
 
 int ag_net_set_engine(ag_net_t* net, int engine) {
     AG_REQUIRE(net != nullptr, "NULL net");
-    AG_REQUIRE(engine == AG_ENGINE_SIMT || engine == AG_ENGINE_TC || engine == AG_ENGINE_TC_EXACT || engine == AG_ENGINE_TC_FAST || engine == AG_ENGINE_TC2 || engine == AG_ENGINE_TC2_BF16, "unknown engine");
+    AG_REQUIRE(engine == AG_ENGINE_SIMT || engine == AG_ENGINE_TC2 || engine == AG_ENGINE_TC2_BF16, "unknown engine");
     AG_REQUIRE(engine != AG_ENGINE_TC2_BF16 || net->kind == AG_NET_HARDNET, "the bf16 engine exists for HardNet only");
-    AG_REQUIRE(engine != AG_ENGINE_TC_FAST || net->kind == AG_NET_AFFNET, "the fast tensor-core engine exists for AffNet only");
-    AG_REQUIRE(engine != AG_ENGINE_TC_EXACT || net->kind != AG_NET_HARDNET, "the exact tensor-core engine exists for AffNet / OriNet");
     net->engine = engine;
     return AG_OK;
 }
@@ -535,8 +506,7 @@ size_t ag_net_workspace_bytes(int kind, int n) {
     const size_t simt = 2 * align_up((size_t)n * per * sizeof(float), 256);
     // tensor-core engine: two fp16 ping-pong buffers + the hi/lo fp16 head operand (AffNet/OriNet, whole 128-patch tiles) or the fp16 head operand (HardNet, padded
     // to a multiple of 128 patches)
-    const size_t act1 = (size_t)n * tc_act_bytes(kind == AG_NET_AFFNET ? AG_NET_ORINET : kind), act2 = tcx_act_bytes(n);   // first / second generation
-    const size_t tcb = 2 * align_up(act1 > act2 ? act1 : act2, 256) +
+    const size_t tcb = 2 * align_up(tcx_act_bytes(n), 256) +
                        (kind == AG_NET_HARDNET ? align_up(((size_t)n + 128) * 8192 * 2, 256) : align_up(tc_headx_bytes(n), 256));
     return simt > tcb ? simt : tcb;
 }
@@ -578,8 +548,7 @@ static int run_trunk(const ag_net* net, const float* patches, const tc::FirstSrc
         // the workspace [a, a + 2*(b-a)) is re-carved as [bufA | bufB | head-GEMM operand]
         char* base = (char*)a;
         const size_t total = 2 * (size_t)((char*)b - (char*)a);
-        const size_t act = net->engine == AG_ENGINE_TC2 ? align_up(tcx_act_bytes(n), 256)
-                                                        : align_up((size_t)n * tc_act_bytes(net->engine == AG_ENGINE_TC_FAST ? net->kind : AG_NET_ORINET), 256);
+        const size_t act = align_up(tcx_act_bytes(n), 256);
         const size_t fbytes = tc_headx_bytes(n);
         if (2 * act + fbytes > total) { set_error("tensor-core workspace too small"); return AG_ERR_CAPACITY; }
         void* bufA = base;
@@ -587,9 +556,7 @@ static int run_trunk(const ag_net* net, const float* patches, const tc::FirstSrc
         b = (float*)(base + 2 * act);
         *feat = b;
         if (net->kind == AG_NET_HARDNET) { set_error("HardNet tensor-core path has its own entry"); return AG_ERR_INVALID; }
-        if (net->engine == AG_ENGINE_TC2) return tcx_trunk_affori(net, src, n, group, count, bufA, bufB, b, st, 6);
-        if (net->engine != AG_ENGINE_TC_FAST) return tc_trunk_orinet(net, src, n, group, count, bufA, bufB, b, st);   // residual planes of weights and activations
-        return tc_trunk_affnet(net, src, n, group, count, bufA, bufB, b, st);
+        return tcx_trunk_affori(net, src, n, group, count, bufA, bufB, b, st, 6);
     }
     *feat = b;
     if (patches == nullptr) { set_error("the fp32 SIMT engine needs materialised patches"); return AG_ERR_INVALID; }
@@ -623,8 +590,8 @@ static int affnet_impl(const ag_net_t* net, const float* d_patches, const tc::Fi
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = run_trunk(net, d_patches, src, n, group, d_count, a, b, &b, st))) return rc;
-    if (net->engine == AG_ENGINE_TC || net->engine == AG_ENGINE_TC_FAST || net->engine == AG_ENGINE_TC2) return tc_headx_forward(net, b, n, group, d_count, d_out, nullptr, st, d_raw);
-    AG_REQUIRE(d_raw == nullptr && d_out, "raw head outputs need a tensor-core engine with the GEMM head (1, 3 or 4)");
+    if (net->engine == AG_ENGINE_TC2) return tc_headx_forward(net, b, n, group, d_count, d_out, nullptr, st, d_raw);
+    AG_REQUIRE(d_raw == nullptr && d_out, "raw head outputs need the tensor-core engine (4)");
     affnet_head_kernel<<<cdiv(n, 8), 256, 0, st>>>(b, net->d_head_w, net->d_head_b, d_out, n, group, d_count);
     AG_CHECK_LAUNCH("affnet_head_kernel");
     return AG_OK;
@@ -641,8 +608,8 @@ static int orinet_impl(const ag_net_t* net, const float* d_patches, const tc::Fi
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = run_trunk(net, d_patches, src, n, group, d_count, a, b, &b, st))) return rc;
-    if (net->engine == AG_ENGINE_TC || net->engine == AG_ENGINE_TC2) return tc_headx_forward(net, b, n, group, d_count, d_out, d_angle, st, d_raw);
-    AG_REQUIRE(d_raw == nullptr, "raw head outputs need a tensor-core engine with the GEMM head (1 or 4)");
+    if (net->engine == AG_ENGINE_TC2) return tc_headx_forward(net, b, n, group, d_count, d_out, d_angle, st, d_raw);
+    AG_REQUIRE(d_raw == nullptr, "raw head outputs need the tensor-core engine (4)");
     orinet_head_kernel<<<cdiv(n, OH_W * OH_P), OH_W * 32, 0, st>>>(b, net->d_head_w, net->d_head_b, d_out, d_angle, n, group, d_count);
     AG_CHECK_LAUNCH("orinet_head_kernel");
     return AG_OK;
@@ -665,12 +632,6 @@ static int hardnet_impl(const ag_net_t* net, const float* d_patches, const tc::F
         const tc::FirstSrc s0 = src ? *src : tc_src_patches(d_patches);
         if ((rc = tcx_trunk_hardnet(net, s0, n, group, d_count, base, base + act, base + 2 * act, st, 6, bf))) return rc;
         return tc_hardnet_head(net, base + 2 * act, n, group, d_count, d_out, st, bf);
-    }
-    if (net->engine == AG_ENGINE_TC) {
-        char* base = (char*)d_ws;
-        const size_t act = align_up((size_t)n * tc_act_bytes(net->kind), 256);
-        const tc::FirstSrc s0 = src ? *src : tc_src_patches(d_patches);
-        return tc_hardnet_forward(net, s0, n, group, d_count, base, base + act, base + 2 * act, d_out, st);
     }
     if ((rc = run_trunk(net, d_patches, src, n, group, d_count, a, b, &b, st))) return rc;
     hardnet_head_kernel<<<cdiv(n, HH_P), 256, 0, st>>>(b, net->d_head_w, net->d_head_b, d_out, n, group, d_count);

@@ -1,7 +1,7 @@
 // Second-generation tensor-core engine of AffNet / OriNet / HardNet (tcx_first.cuh, tcx_conv.cuh): row tiles without x padding, the
 // three taps of a kernel row stacked along N, x shifts by warp shuffles in the epilogue.  Replaces the conv stacks of
-// architectures.py:207-235 / 36-82 and HardNet.py:67-101 (BatchNorm folded, ReLU fused); the 8x8 heads stay the GEMM kernels of
-// tc_head.cuh (same head-operand layout).  Per net:  tcx_first_kernel (sampler + input_norm + conv1 + conv2)  ->  tcx_conv_kernel x4;
+// architectures.py:207-235 / 36-82 and HardNet.py:67-101 (BatchNorm folded, ReLU fused); the 8x8 heads are the GEMM kernels of
+// tc_head.cuh (tc_head_kernel, tc_headx_kernel).  Per net:  tcx_first_kernel (sampler + input_norm + conv1 + conv2)  ->  tcx_conv_kernel x4;
 // AffNet / OriNet: conv3 inside tcx_first_kernel as well (AG_FUSE_L3), then tcx_conv_kernel x3.
 // Numerics: AffNet / OriNet with fp16 residual planes of weights and activations in every layer (three MMAs per K step, fp32-grade);
 // HardNet fp16 activations, weights with their fp16 residual in layers 2 and 3 (emulation on the 2000 graf patches: plain fp16 weights give a
@@ -15,6 +15,7 @@
 #include <cuda_bf16.h>
 
 #include "net_impl.cuh"
+#include "tc_head.cuh"
 #include "tcx_conv.cuh"
 #include "tcx_first.cuh"
 
@@ -115,6 +116,62 @@ __global__ void tcx_decode_kernel(const __half* __restrict__ buf, int layout, in
 }
 
 }  // namespace tcx
+
+// ---- sources of the first kernel: materialised patches, or the pyramid + keypoints ---------------------------------------------------
+tc::FirstSrc tc_src_patches(const float* patches) {
+    tc::FirstSrc s;
+    memset(&s, 0, sizeof(s));
+    s.patches = patches;
+    s.cap = 1;
+    return s;
+}
+
+tc::FirstSrc tc_src_pyramid(const ag_pyramid_plan_t* p, const float* pyr, const float* lafs, const int* oct, const int* lvl, int cap) {
+    tc::FirstSrc s;
+    memset(&s, 0, sizeof(s));
+    s.pyr = pyr; s.lafs = lafs; s.oct = oct; s.lvl = lvl; s.cap = cap;
+    s.geom.n_octaves = p->n_octaves; s.geom.n_levels = p->n_levels;
+    for (int o = 0; o < AG_MAX_OCTAVES; o++) {
+        s.geom.h[o] = p->h[o]; s.geom.w[o] = p->w[o];
+        for (int l = 0; l < AG_MAX_LEVELS; l++) s.geom.off[o][l] = p->level_offset[o][l];
+    }
+    return s;
+}
+
+// ---- heads ----------------------------------------------------------------------------------------------------------------------------
+// HardNet 8x8 head GEMM + BatchNorm + L2 norm over the head operand a trunk left in `headbuf`
+int tc_hardnet_head(const ag_net* net, const void* headbuf, int n, int group, const int* count, float* out, cudaStream_t st, int bf16) {
+    using namespace tc;
+    static SmemAttrOnce once0, once1;
+    {
+        int rc = once0.ensure(tc_head_kernel<0>, HEAD_SMEM, "tc_head smem attr");
+        if (rc == AG_OK) rc = once1.ensure(tc_head_kernel<1>, HEAD_SMEM, "tc_head smem attr");
+        if (rc != AG_OK) return rc;
+    }
+    if (bf16) tc_head_kernel<1><<<(n + 127) / 128, 192, HEAD_SMEM, st>>>((const __half*)headbuf, net->d_headh_bf, net->d_head_b, out, n, group, count);
+    else tc_head_kernel<0><<<(n + 127) / 128, 192, HEAD_SMEM, st>>>((const __half*)headbuf, net->d_headh, net->d_head_b, out, n, group, count);
+    AG_CHECK_LAUNCH("tc_head_kernel");
+    return AG_OK;
+}
+
+// AffNet / OriNet head on tensor cores over the hi/lo feature planes the trunk leaves in `feat`
+int tc_headx_forward(const ag_net* net, const void* feat, int n, int group, const int* count, float* out, float* angle, cudaStream_t st, float* raw) {
+    using namespace tc;
+    static SmemAttrOnce once0, once1;
+    {
+        int rc = once0.ensure(tc_headx_kernel<0>, HX_SMEM, "tc_headx smem attr");
+        if (rc == AG_OK) rc = once1.ensure(tc_headx_kernel<1>, HX_SMEM, "tc_headx smem attr");
+        if (rc != AG_OK) return rc;
+    }
+    const int tiles = (n + 127) / 128;
+    if (net->kind == AG_NET_AFFNET) tc_headx_kernel<0><<<tiles, 192, HX_SMEM, st>>>((const __half*)feat, net->d_headh, net->d_head_b, net->head_inv_scale, out, nullptr, raw, n, group, count);
+    else tc_headx_kernel<1><<<tiles, 192, HX_SMEM, st>>>((const __half*)feat, net->d_headh, net->d_head_b, net->head_inv_scale, out, angle, raw, n, group, count);
+    AG_CHECK_LAUNCH("tc_headx_kernel");
+    return AG_OK;
+}
+
+// bytes of the head-GEMM operand of n patches (hi + lo planes, padded to whole 128-patch tiles)
+size_t tc_headx_bytes(int n) { return (size_t)((n + 127) / 128) * 2 * tc::HX_PLANE_TILE; }
 
 // ---- weight packing (host) --------------------------------------------------------------------------------------------------------
 // wf: fp32 [tap = dy*3+dx][ci][co] (BatchNorm folded), scale: power of two.  Blocks per (split, dy, 16 input channels):

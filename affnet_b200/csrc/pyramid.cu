@@ -14,7 +14,6 @@
 #include <cuda.h>   // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint, libcuda is not linked)
 
 #include "common.cuh"
-#include "pyramid_fused.cuh"
 
 namespace ag {
 
@@ -288,64 +287,6 @@ static int launch_blur(const float* in, float* out, float* dec, int B, int h, in
     return AG_OK;
 }
 
-static int g_pyr_fused = 0;   // developer switch, see ag_pyramid_build
-
-// ---- one launch per octave (pyramid_fused.cuh) ---------------------------------------------------------------------------------
-static int num_sms_pyr() {
-    static int n = 0;
-    if (n == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        if (n <= 0) n = 148;
-    }
-    return n;
-}
-
-// The fused kernel is specialised for the reference's only configuration (nlevels = 3, init_sigma = 1.6: radii 5 | 4 5 6 7) and rows
-// whose length is a multiple of four floats; anything else takes the per-level launches.
-template <int CH>
-static int launch_octave(const float* src, float* const* outs, float* dec, int seed, int B, int h, int w, const double* sigmas, cudaStream_t st, bool* handled) {
-    using C = pf::Chain<CH>;
-    *handled = false;
-    if ((w & 3) != 0 || w < 8 || h < 2) return AG_OK;
-    if ((reinterpret_cast<size_t>(src) & 15) || (dec && (reinterpret_cast<size_t>(dec) & 15))) return AG_OK;   // 128-bit rows / bulk copies
-    for (int l = 0; l < C::NB; l++)
-        if (reinterpret_cast<size_t>(outs[l]) & 15) return AG_OK;
-    pf::OctArgs a;
-    memset(&a, 0, sizeof(a));
-    for (int l = 0; l < C::NB; l++) {
-        BlurTaps t;
-        int rc = make_taps(sigmas[l], &t);
-        if (rc != AG_OK) return rc;
-        if (t.r != C::R(l)) return AG_OK;      // another sigma schedule: not this specialisation
-        for (int k = 0; k <= 2 * t.r; k++) a.taps[l][k] = t.w[k];
-        a.out[l] = outs[l];
-    }
-    a.src = src; a.dec = dec; a.seed = seed; a.B = B; a.h = h; a.w = w;
-    a.nstrips = cdiv(w, pf::SWMAX);
-    a.sw = cdiv(cdiv(w, a.nstrips), 4) * 4;
-    a.nstrips = cdiv(w, a.sw);
-    int nb = (2 * num_sms_pyr() + a.nstrips * B - 1) / (a.nstrips * B);     // about two CTAs per SM ...
-    const int nb_max = h / 48 > 1 ? h / 48 : 1;                              // ... but bands of at least 48 rows (a band re-computes up to 27 rows of warm-up)
-    if (nb > nb_max) nb = nb_max;
-    if (nb < 1) nb = 1;
-    a.band = cdiv(h, nb);
-    a.nbands = cdiv(h, a.band);
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!configured[dev & 63]) {
-        int rc = check_cuda(cudaFuncSetAttribute(pf::octave_kernel<CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(pf::Smem<CH>)), "octave smem attr");
-        if (rc != AG_OK) return rc;
-        configured[dev & 63] = true;
-    }
-    pf::octave_kernel<CH><<<dim3(a.nstrips * a.nbands, B), 64 * C::NB, sizeof(pf::Smem<CH>), st>>>(a);
-    AG_CHECK_LAUNCH("octave_kernel");
-    *handled = true;
-    return AG_OK;
-}
-
 __global__ void decimate_kernel(const float* __restrict__ in, float* __restrict__ out, int h, int w, int h2, int w2) {
     int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y, b = blockIdx.z;
     if (x < w2) out[(size_t)b * h2 * w2 + (size_t)y * w2 + x] = in[(size_t)b * h * w + (size_t)(2 * y) * w + 2 * x];
@@ -429,12 +370,6 @@ int ag_pyramid_plan(int B, int H, int W, int nlevels, double init_sigma, int bor
     return AG_OK;
 }
 
-int ag_debug_pyramid_mode(int fused) {
-    const int old = g_pyr_fused;
-    g_pyr_fused = fused ? 1 : 0;
-    return old;
-}
-
 int ag_gaussian_blur(const float* d_in, float* d_out, int B, int h, int w, double sigma, void* stream) {
     AG_REQUIRE(d_in && d_out && B >= 1 && h >= 1 && w >= 1, "bad arguments");
     return launch_blur(d_in, d_out, nullptr, B, h, w, sigma, (cudaStream_t)stream);
@@ -444,33 +379,10 @@ int ag_pyramid_build(const ag_pyramid_plan_t* p, const float* d_img, float* d_py
     AG_REQUIRE(p && d_img && d_pyr, "NULL argument");
     cudaStream_t st = (cudaStream_t)stream;
     const int nl = p->n_levels, seed_level = nl - 2;  // level `nlevels` seeds the next octave (:46-47)
-    // Measured (r02, 16 x 1024x768): the one-launch-per-octave kernel is bit-identical but SLOWER than the per-level launches (octave 0: 0.80
-    // vs 0.26 ms, whole pyramid 1.35 vs 0.68 ms): both are bound by instruction issue, and streaming rows gives the vertical pass one
-    // 128-bit shared-memory load per 4 FMAs where blur_kernel's 4x4 register block gets 16.  It stays selectable for A/B runs
-    // (ag_debug_pyramid_mode(1) or AG_PYR_FUSED=1); the default is the per-level path.
-    static const bool env_fused = getenv("AG_PYR_FUSED") != nullptr;
-    const bool no_fused = !(env_fused || g_pyr_fused);
+    // One launch per level: a one-launch-per-octave kernel was measured bit-identical but 2x slower (DESIGN.md section 5).
     for (int o = 0; o < p->n_octaves; o++) {
         const int h = p->h[o], w = p->w[o];
         float* lvl0 = d_pyr + p->level_offset[o][0];
-        float* next0 = (o + 1 < p->n_octaves) ? d_pyr + p->level_offset[o + 1][0] : nullptr;
-        if (nl == 5 && !no_fused) {   // one launch for the whole octave
-            bool handled = false;
-            int rc;
-            if (o == 0 && p->blur_sigma[0][0] > 0.0) {
-                float* outs[5];
-                double sg[5];
-                for (int l = 0; l < 5; l++) { outs[l] = d_pyr + p->level_offset[0][l]; sg[l] = p->blur_sigma[0][l]; }
-                rc = launch_octave<0>(d_img, outs, next0, seed_level, p->B, h, w, sg, st, &handled);
-            } else if (o > 0) {
-                float* outs[4];
-                double sg[4];
-                for (int l = 1; l < 5; l++) { outs[l - 1] = d_pyr + p->level_offset[o][l]; sg[l - 1] = p->blur_sigma[o][l]; }
-                rc = launch_octave<1>(lvl0, outs, next0, seed_level - 1, p->B, h, w, sg, st, &handled);
-            } else rc = AG_OK;
-            if (rc != AG_OK) return rc;
-            if (handled) continue;
-        }
         if (o == 0) {
             if (p->blur_sigma[0][0] > 0.0) {
                 int rc = launch_blur(d_img, lvl0, nullptr, p->B, h, w, p->blur_sigma[0][0], st);

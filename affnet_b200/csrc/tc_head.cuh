@@ -1,10 +1,10 @@
 // HardNet 8x8 head on tensor cores: conv8x8(128->128, no bias) == GEMM [n, 8192] x [8192, 128], then BatchNorm and
-// L2 normalisation (HardNet.py:86-101, 12-19).  A = trunk features in the HEADL layout written by the last conv layer
+// L2 normalisation (HardNet.py:86-101, 12-19).  A = trunk features in the L_HEAD layout written by the last conv layer
 // ([patch/128][k/8][patch%128][8] fp16: 128 patches are the M rows of one tile), B = head weights [k/8][cout][8] fp16.
 // One CTA per 128-patch tile streams K in 64-wide stages (A 16 KiB + B 16 KiB per stage, bulk copies, 6-stage ring),
 // accumulates 128x128 fp32 in TMEM, and the epilogue thread of each row does BN + sum of squares + scale in registers.
 #pragma once
-#include "tc_conv.cuh"
+#include "tcgen05.cuh"
 
 namespace ag {
 namespace tc {
@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(192, 1) tc_head_kernel(const __half* __restric
 
 // ---- AffNet / OriNet heads on tensor cores -------------------------------------------------------------------------------
 // conv8x8(64 -> 3) resp. the padded conv8x8(64 -> 2) seen as 18 shifted dot products (nets_simt.cu) == GEMM [n, 4096] x
-// [4096, 32] with fp32-grade operands: the last conv layer writes its output as fp16 hi + lo planes in the HEADL layout, the head
+// [4096, 32] with fp32-grade operands: the last conv layer writes its output as fp16 hi + lo planes in the L_HEAD layout, the head
 // weights are stored as [k/8][W_hi rows 0..31 | W_lo rows 32..63][8], and per K step the issuer runs A_hi x [W_hi ; W_lo]
 // (N = 64) and A_lo x W_hi (N = 32); the epilogue adds the two accumulator halves and applies the reference's post-processing
 // (architectures.py:57-59,76-82,228-230; LAF.py:276-291).  One CTA per 128-patch tile, K streamed in 64-wide stages.

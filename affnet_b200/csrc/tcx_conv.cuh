@@ -2,8 +2,8 @@
 // stacked along N.
 //
 // Measured on B200 (tests/probe/tc_rates.cu): one tcgen05.mma kind::f16 (M = 128, K = 16) costs max(47.5, N/2) clk whatever its
-// operands' source, so an MMA with N = 16 .. 64 leaves 66 - 90 % of the tensor pipe idle.  The first-generation engine (tc_conv.cuh)
-// issued one MMA per tap (N = 16 .. 64); here the three taps of a kernel ROW share one MMA:
+// operands' source, so an MMA with N = 16 .. 64 leaves 66 - 90 % of the tensor pipe idle.  One MMA per tap (N = 16 .. 64, the
+// formulation of the first-generation engine, DESIGN.md section 4) is therefore avoided; here the three taps of a kernel ROW share one MMA:
 //
 //   pixel planes are stored WITHOUT x padding, so that an M = 128 tile is 128 consecutive pixels = whole image rows (4 rows of 32,
 //   8 rows of 16, or 8 rows of 8 of TWO patches interleaved row by row), and every warp of the epilogue owns whole rows;
@@ -31,7 +31,7 @@
 #pragma once
 #include <cuda_bf16.h>
 
-#include "tc_conv.cuh"
+#include "tcgen05.cuh"
 
 namespace ag {
 namespace tcx {

@@ -163,26 +163,21 @@ typedef struct ag_net ag_net_t;
 int ag_net_create(int kind, const float* h_blob, size_t n_floats, ag_net_t** out);
 void ag_net_destroy(ag_net_t* net);
 size_t ag_net_blob_floats(int kind);
-/* Compute engine: 0 = exact fp32 SIMT (needs materialised patches); 1 = first-generation tcgen05 engine (round 1; one MMA per tap): fp16
- * operands, fp32 accumulation in TMEM, all six conv layers and the 8x8 heads as MMAs; AffNet and OriNet carry fp16 residual
- * planes of weights AND activations in every layer (fp32-grade: A 1e-5, angle 3e-5 rad - OriNet's atan2 amplifies an error of
- * AffNet's A about 15x, so the 1e-3 LAF contract needs A to 5e-5), HardNet plain fp16 operands (descriptors 6e-4);
- * 2 = as 1 with fp32 FMA-chain heads (A 2e-6, angle 3e-6 rad; AffNet/OriNet only); 3 = AffNet with the weight residual only
- * (A 2e-4; for A/B timing, AffNet only);
- * 4 = second-generation tcgen05 engine, THE DEFAULT for all three nets (same operand precision as 1, plus fp16 residuals of HardNet's
- * layer 2-3 weights: descriptors 4e-4): 128-pixel
- * row tiles without x padding, the three taps of a kernel row stacked along N of one MMA, x shifts by warp shuffles in the epilogue;
- * 5 = engine 4 with bf16 operands (HardNet only; BASELINE.json configs[4] "bf16 HardNet tensor-core path"; descriptors ~4e-3). */
+/* Compute engine: 0 = exact fp32 SIMT (needs materialised patches);
+ * 4 = tcgen05 tensor-core engine, THE DEFAULT for all three nets: fp16 operands, fp32 accumulation in TMEM, all six conv layers and the
+ * 8x8 heads as MMAs; 128-pixel row tiles without x padding, the three taps of a kernel row stacked along N of one MMA, x shifts by warp
+ * shuffles in the epilogue.  AffNet and OriNet carry fp16 residual planes of weights AND activations in every layer (fp32-grade: A 1e-5,
+ * angle 3e-5 rad - OriNet's atan2 amplifies an error of AffNet's A about 15x, so the 1e-3 LAF contract needs A to 5e-5); HardNet fp16
+ * activations with fp16 residuals of its layer 2-3 weights (descriptors 4e-4);
+ * 5 = engine 4 with bf16 operands (HardNet only; BASELINE.json configs[4] "bf16 HardNet tensor-core path"; descriptors ~4e-3).
+ * Engines 1, 2 and 3 (the first-generation tensor-core engine and its variants) no longer exist and are refused with AG_ERR_INVALID. */
 int ag_net_set_engine(ag_net_t* net, int engine);
 int ag_net_get_engine(const ag_net_t* net);
-/* Developer switch: 1 = ag_pyramid_build runs one launch per octave (pyramid_fused.cuh: bit-identical, measured slower), 0 = one
- * launch per level (default).  Returns the previous mode. */
-int ag_debug_pyramid_mode(int fused);
 /* Developer switch: 1 = conv layer 3 of AffNet / OriNet runs inside the first tcgen05 kernel (layer 2's output stays in shared memory;
  * bit-identical; the default unless built with -DAG_FUSE_L3=0), 0 = first kernel and layer-3 kernel as two launches.  Returns the
  * previous mode. */
 int ag_debug_fuse_l3(int fused);
-/* Developer diagnostic: run the second-generation trunk on materialised patches [n,32,32] up to conv layer `upto` (2..5) and decode
+/* Developer diagnostic: run the tensor-core trunk on materialised patches [n,32,32] up to conv layer `upto` (2..5) and decode
  * that layer's activations (fp16 hi [+ lo] planes in the engine's HBM layout) to fp32 [n,C,H,H].  d_ws: ag_net_workspace_bytes(). */
 int ag_debug_tcx_layer(const ag_net_t* net, const float* d_patches, int n, int upto, float* d_out, void* d_ws, size_t ws_bytes, void* stream);
 /* Scratch bytes for a forward over n patches. */
@@ -203,7 +198,7 @@ int ag_hardnet_forward(const ag_net_t* net, const float* d_patches, int n, const
 /* f4: the TorchScript exports' contract (convertJIT/AffNetJIT.pt, OriNetJIT.pt; convert_OriNet_and_AffNet_to_JIT.ipynb): the RAW head
  * outputs.  AffNet: xy + [1, 0, 1] = (1 + x0, x1, 1 + x2) -> d_raw [n,3] (architectures.py:228-230 before rectification);
  * OriNet: the mean over the 3x3 map of tanh(conv8x8) -> d_raw [n,2] = (sin-like, cos-like) (architectures.py:57-59,76).
- * Tensor-core engines only (1, 3, 4). */
+ * Tensor-core engine (4) only. */
 int ag_affnet_forward_raw(const ag_net_t* net, const float* d_patches, int n, float* d_raw, void* d_ws, size_t ws_bytes, void* stream);
 int ag_orinet_forward_raw(const ag_net_t* net, const float* d_patches, int n, float* d_raw, void* d_ws, size_t ws_bytes, void* stream);
 /* Fused sampler + net (tensor-core engine): LAF i of image b is sampled at pyr[oct][lvl] INSIDE the first tensor-core

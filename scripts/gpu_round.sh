@@ -12,7 +12,7 @@ tail -c 3000 gpurun_out/bench.json; tail -5 gpurun_out/bench.err
 if [ "${SKIP_NCU:-0}" != "1" ]; then
 ncu --metrics gpu__time_duration.sum --clock-control none -c 500 --csv --log-file gpurun_out/launches.csv \
     python bench.py --steps 1 --warmup 3 --batch 4 --no-cpu-baseline --no-graph > gpurun_out/ncu_bench.log 2>&1
-ncu --set full --clock-control none --import-source on --kernel-name-base demangled -k "regex:${NCU_KERNEL:-tc_conv_kernel}" -s ${NCU_SKIP:-0} -c ${NCU_COUNT:-3} \
+ncu --set full --clock-control none --import-source on --kernel-name-base demangled -k "regex:${NCU_KERNEL:-tcx_conv_kernel}" -s ${NCU_SKIP:-0} -c ${NCU_COUNT:-3} \
     -o gpurun_out/prof_top -f python bench.py --steps 1 --warmup 3 --batch 2 --no-cpu-baseline --no-graph > gpurun_out/ncu_full.log 2>&1
 ls -la gpurun_out
 fi

@@ -1,6 +1,6 @@
-"""GPU tests of the second-generation tensor-core engine (ENGINE_TC2, tcx_first.cuh / tcx_conv.cuh): every conv layer's activations
-against the fp32 oracle (stage-isolated: `ag_debug_tcx_layer` decodes the engine's HBM layout), the three nets end to end, and
-tile / pair / persistent-stride invariance."""
+"""GPU tests of the tensor-core engine (ENGINE_TC2, tcx_first.cuh / tcx_conv.cuh): every conv layer's activations against the fp32
+oracle (stage-isolated: `ag_debug_tcx_layer` decodes the engine's HBM layout), the three nets end to end, tile / pair / persistent-stride
+invariance, and the engine selection."""
 import ctypes as C
 
 import numpy as np
@@ -88,16 +88,17 @@ def test_tcx_nets_vs_oracle(L, nets):
     sets = [torch.from_numpy(z["aff_patches"]), torch.from_numpy(z["ori_desc_patches"]), torch.rand(37, 1, 32, 32, generator=g) * 255,
             torch.from_numpy(gold("face_patches.npz")["patches_u8"].astype(np.float32) / 255.0).view(-1, 1, 32, 32),
             torch.rand(300, 1, 32, 32, generator=g)]
-    worst = [0.0, 0.0, 0.0]
+    worst = [0.0, 0.0, 0.0, 0.0]
     for P in sets:
         Pd = P.to(DEV)
         dA = (aff(Pd).cpu() - O.affnet_forward(P, W["affnet"])).abs().max().item()
+        dR = (ori(Pd).cpu() - O.orinet_forward(P, W["orinet"])).abs().max().item()
         dang = (ori(Pd, return_rot_matrix=False).cpu() - O.orinet_angle(P, W["orinet"]))
         dang = torch.atan2(torch.sin(dang), torch.cos(dang)).abs().max().item()
         dD = (hn(Pd).cpu() - O.hardnet_forward(P, W["hardnet"])).abs().max().item()
-        worst = [max(a, b) for a, b in zip(worst, (dA, dang, dD))]
-    print("\nengine tc2: max|dA| %.2e  max|dangle| %.2e rad  max|ddesc| %.2e" % tuple(worst))
-    assert worst[0] < 5e-5 and worst[1] < 1e-4 and worst[2] < 6e-4, worst
+        worst = [max(a, b) for a, b in zip(worst, (dA, dR, dang, dD))]
+    print("\nengine tc2: max|dA| %.2e  max|dR| %.2e  max|dangle| %.2e rad  max|ddesc| %.2e" % tuple(worst))
+    assert worst[0] < 5e-5 and worst[1] < 1e-4 and worst[2] < 1e-4 and worst[3] < 6e-4, worst
 
 
 def test_tcx_batching_invariance(L, nets):
@@ -125,10 +126,29 @@ def test_raw_heads_vs_reference_torchscript(L):
     print("\nraw heads vs TorchScript goldens: AffNet %.2e, OriNet %.2e" % (da, do))
     assert a(P).shape == (P.size(0), 3) and o(P).shape == (P.size(0), 2)
     assert da < 2e-5 and do < 2e-5
-    for eng in (L.ENGINE_TC,):      # first-generation engine: same entry points
-        a.set_engine(eng); o.set_engine(eng)
-        assert (a(P).cpu() - torch.from_numpy(z["affnet_raw"])).abs().max() < 2e-5
-        assert (o(P).cpu() - torch.from_numpy(z["orinet_raw"])).abs().max() < 2e-5
+
+
+def test_engine_selection(L, nets):
+    """Engines 1, 2 and 3 (the first-generation tensor-core engine and its variants) do not exist: ag_net_set_engine refuses them and
+    leaves the net's engine as it was.  0 (SIMT), 4 (tensor cores) and, for HardNet, 5 (bf16) select and run."""
+    P = patches()[:40].to(DEV)
+    for m in nets:
+        ref = m(P)
+        try:
+            for e in (1, 2, 3):
+                with pytest.raises(L.AffnetB200Error):
+                    m.set_engine(e)
+                assert m.engine == L.ENGINE_TC2
+            engines = (L.ENGINE_SIMT, L.ENGINE_TC2, L.ENGINE_TC2_BF16) if m.KIND == L.NET_HARDNET else (L.ENGINE_SIMT, L.ENGINE_TC2)
+            for e in engines:
+                m.set_engine(e)
+                assert m.engine == e
+                assert (m(P) - ref).abs().max().item() < 1e-2, (type(m).__name__, e)
+            if m.KIND != L.NET_HARDNET:
+                with pytest.raises(L.AffnetB200Error):
+                    m.set_engine(L.ENGINE_TC2_BF16)
+        finally:
+            m.set_engine(L.ENGINE_TC2)
 
 
 def test_hardnet_bf16_engine(L):

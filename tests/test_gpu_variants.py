@@ -46,7 +46,7 @@ torch.save({"pyr": buf.cpu(), "resp": resp.cpu(), "lafs": lafs.cpu(), "oc": oc.c
 def _run(tmp_path, name, env_extra):
     out = str(tmp_path / (name + ".pt"))
     env = dict(os.environ)
-    for k in ("AG_BLUR_NO_TMA", "AG_DETECT_WARP_V1", "AG_PYR_FUSED"):
+    for k in ("AG_BLUR_NO_TMA", "AG_DETECT_WARP_V1"):
         env.pop(k, None)
     env.update(env_extra)
     r = subprocess.run([sys.executable, "-c", _SCRIPT, out, ROOT], env=env, capture_output=True, text=True, timeout=600)
